@@ -191,6 +191,26 @@ def ray_parity(out, rm_cls, dev):
             'oracle_miou_vs_gt_scene': float(g['miou']), 'frame': 'seed 100 (the golden frame)'}
 
 
+DUMP_BYTES = 60 * 10**6                                             # data of all files; stays under 64 MB with the headers
+
+
+def dump_outputs(outs, path):
+    """The last timed step's engine outputs -> <path>/<name>.npy in float32, stacked over the step's frames:
+    (frames, X, Y, Z[, 2]).  Above DUMP_BYTES in all, every frame keeps the same seeded sample of voxels (row-major
+    (X, Y, Z) order): (frames, voxels[, 2])."""
+    os.makedirs(path, exist_ok=True)
+    names = sorted(outs[0])
+    nvox = int(np.prod(outs[0][names[0]].shape[:3]))                # every output is (X, Y, Z, ...)
+    per_voxel = sum(outs[0][k].numel() // nvox for k in names) * 4 * len(outs)
+    idx = None
+    if per_voxel * nvox > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(nvox, DUMP_BYTES // per_voxel, replace=False))
+        idx = torch.from_numpy(idx).to(outs[0][names[0]].device)
+    for k in names:
+        a = torch.stack([o[k] if idx is None else o[k].flatten(0, 2)[idx] for o in outs]).float()
+        np.save(os.path.join(path, k + '.npy'), a.cpu().numpy())
+
+
 def timed_region(run_steps, steps, barrier):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
@@ -232,9 +252,14 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last_step = []                                                  # --dump-outputs: outputs of the last step run
+
     def run_steps(n):                                               # one step = F frames through the engine
+        last_step.clear()
         for i in range(n * F):
-            eng.forward(frames_dev[i % NF], want=want)
+            out = eng.forward(frames_dev[i % NF], want=want)
+            if args.dump_outputs and i >= (n - 1) * F:
+                last_step.append(out)
 
     # ---- device-resident throughput (`value`): >= 1 s of warm-up, then `repeats` regions of EXACTLY K steps, median
     run_steps(W)
@@ -248,6 +273,8 @@ def run_ours(args):
         sampler.start()
     reps = [occdist.max_over_ranks(timed_region(run_steps, K, barrier), dev) for _ in range(args.repeats)]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last_step, args.dump_outputs)
     ms_med = float(np.median(reps))
     launches = eng.launches_per_frame
 
@@ -735,6 +762,8 @@ def main():
     ap.add_argument('--frames-per-step', type=int, default=32, help='one step = this many frames through the engine')
     ap.add_argument('--repeats', type=int, default=3, help='timed regions (each exactly --steps steps); median reported')
     ap.add_argument('--no-backbone', action='store_true', help='skip the images -> ResNet-50+FPN -> hot path leg')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (rank 0) as DIR/<name>.npy, float32 (see dump_outputs)')
     args = ap.parse_args()
     if args.impl == 'reference':
         run_reference(args)

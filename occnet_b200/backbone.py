@@ -23,12 +23,12 @@ class BackboneEngine:
     """state_dict: the detector's `state_dict()` (or any mapping holding its img_backbone.* / img_neck.* entries)."""
 
     def __init__(self, state_dict, num_images, img_hw, precision='fp32', use_tensor_cores=None, device='cuda:0'):
-        if not torch.cuda.is_available():
+        self.device = torch.device(device)
+        if not torch.cuda.is_available() or self.device.type != 'cuda':
             raise RuntimeError('libocc_b200 backbone needs a CUDA device (there is no CPU path)')
         assert precision in ('fp32', 'bf16')
         self.lib = _lib.load()
         self.precision = precision
-        self.device = torch.device(device)
         self.num_images, (self.H, self.W) = int(num_images), (int(img_hw[0]), int(img_hw[1]))
         tc = (precision == 'bf16') if use_tensor_cores is None else bool(use_tensor_cores)
         with torch.cuda.device(self.device):

@@ -5,8 +5,9 @@ dvr.cu does not compile against torch 2.11 as shipped (`AT_DISPATCH_FLOATING_TYP
 dvr.cu:371,683,736), so the recipe compiles a scratch copy under /tmp with the 3-token fix
 `.type()` -> `.scalar_type()` applied by sed.  Nothing from the reference is copied into the repository;
 only the built `dvr_ref.so` lands in oracle/_ref/ (git-ignored, travels to the GPU box).
-The GPU test tests/test_gpu_parity.py::test_render_forward_vs_reference_kernel_if_built uses it to pin
-both the CUDA ray-caster and the C restatement (oracle/ray_dda.c) against the reference kernel itself.
+tests/golden/gen_dvr_ref.py runs it on a GPU and stores its outputs in tests/golden/ref_dvr.npz, against which
+tests/test_gpu_parity.py::test_render_forward_vs_reference_kernel pins both the CUDA ray-caster and the C restatement
+(oracle/ray_dda.c).
 """
 import os
 import re

@@ -193,7 +193,20 @@ def gen_metric_golden():
     print('[metric] wrote ref_metric.npz; miou', fin['miou'], 'mave', fin['mave'])
 
 
+def gen_config_golden():
+    """The shipped config as `Config.fromfile` loads it (`_base_` files merged), reduced to the keys the drop-in tests
+    read: plugin, plugin_dir, dist_params and the model."""
+    import json
+    cfg = mmcv_shim.Config.fromfile(os.path.join(REF, 'projects', 'configs', 'bevformer', 'bevformer_base_occ.py'))
+    keep = {k: cfg[k] for k in ('plugin', 'plugin_dir', 'dist_params', 'model')}
+    with open(os.path.join(OUT, 'ref_config_base_occ.json'), 'w') as f:
+        json.dump(keep, f, indent=1)
+        f.write('\n')
+    print('[config] wrote ref_config_base_occ.json')
+
+
 if __name__ == '__main__':
     mods = import_reference()
     gen_model_goldens(mods)
     gen_metric_golden()
+    gen_config_golden()

@@ -1,4 +1,5 @@
 """CPU suite: the drop-in surface (config loading, registries, state_dict key contract) and the data-parallel host logic."""
+import json
 import os
 import subprocess
 import sys
@@ -11,10 +12,21 @@ from occnet_b200 import fixtures
 from occnet_b200.mmcv_shim import Config, build_detector, build_head
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_CFG = '/root/reference/projects/configs/bevformer/bevformer_base_occ.py'
 
 
 head_cfg = fixtures.head_cfg          # registry config of the head for a fixture geometry (shared with bench.py)
+
+
+def shipped_config(golden_dir, tmp_path):
+    """The reference's projects/configs/bevformer/bevformer_base_occ.py, reduced to plugin, plugin_dir, dist_params and
+    model (written by tests/golden/gen_golden.py), laid out again as the shipped files are -- dist_params in a
+    `_base_` runtime file, the rest in the config that inherits it -- and loaded through `Config.fromfile`."""
+    with open(os.path.join(golden_dir, 'ref_config_base_occ.json')) as f:
+        d = json.load(f)
+    (tmp_path / 'default_runtime.py').write_text(f"dist_params = {d.pop('dist_params')!r}\n")
+    path = tmp_path / 'bevformer_base_occ.py'
+    path.write_text("_base_ = ['default_runtime.py']\n" + ''.join(f'{k} = {v!r}\n' for k, v in d.items()))
+    return Config.fromfile(str(path))
 
 
 def test_plugin_state_dict_keys_equal_reference(golden_dir):
@@ -28,10 +40,9 @@ def test_plugin_state_dict_keys_equal_reference(golden_dir):
     head.load_state_dict(fixtures.init_params(cfg, seed=2), strict=True)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason='reference tree not present (GPU box)')
-def test_shipped_config_loads_and_builds_unchanged():
+def test_shipped_config_loads_and_builds_unchanged(golden_dir, tmp_path):
     import projects.mmdet3d_plugin  # noqa: F401
-    cfg = Config.fromfile(REF_CFG)
+    cfg = shipped_config(golden_dir, tmp_path)
     assert cfg.plugin and cfg.plugin_dir == 'projects/mmdet3d_plugin/'
     assert cfg.model.type == 'BEVFormerOcc' and cfg.dist_params.backend == 'nccl'          # `_base_` merge works
     assert cfg.model.pts_bbox_head.transformer.encoder.num_layers == 4
@@ -45,15 +56,14 @@ def test_shipped_config_loads_and_builds_unchanged():
         head([torch.zeros(1, 6, 256, h, w) for h, w in fixtures.CFG_FULL['level_shapes']], fixtures.make_img_metas(fixtures.CFG_FULL))
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason='reference tree not present (GPU box)')
-def test_backbone_neck_containers_have_reference_keys():
+def test_backbone_neck_containers_have_reference_keys(golden_dir, tmp_path):
     """img_backbone / img_neck of the shipped config build as parameter containers whose keys are the reference's
     (mmdet ResNet == torchvision resnet50 minus fc; mmdet FPN lateral_convs / fpn_convs) and accept the oracle's
     parameter dict unchanged."""
     import projects.mmdet3d_plugin  # noqa: F401
     from torchvision.models import resnet50
     from oracle import backbone as OB
-    det = build_detector(Config.fromfile(REF_CFG).model)
+    det = build_detector(shipped_config(golden_dir, tmp_path).model)
     sd = det.state_dict()
     bk = {k[len('img_backbone.'):] for k in sd if k.startswith('img_backbone.')}
     assert bk == {k for k in resnet50(weights=None).state_dict() if not k.startswith('fc.')}

@@ -12,8 +12,6 @@
 //   warp 0: TMA producer (8-stage ring)    warp 1: tcgen05.mma issuer (plane-major: each loaded tile feeds the
 //   dx = 0/1/2 taps of three neighbouring outputs through ONE N = 96 MMA into adjacent TMEM slots, ring of 8)
 //   warps 2-5: epilogue (tcgen05.ld -> +bias -> ReLU -> bf16 -> 64-byte rows, contiguous 8 KB per tile)
-#include <cstdlib>
-
 #include "common.cuh"
 #include "conv3d_tc.cuh"
 #include "tc_common.cuh"
@@ -37,15 +35,15 @@ constexpr int BAR_BYTES = 512;
 // accumulates and the issue loop has no per-output special cases.
 // Each CTA owns a contiguous range of the (y_tile, x) tile sequence, cut into segments of constant y_tile; a segment
 // [xa, xb) streams the planes max(xa-1,0) .. min(xb, X-1).
-// UNI: the producer / issuer warps run their loops with ALL 32 lanes (lane 0 alone executes the TMA / MMA / commit
-// instructions): loop counters, stage indices and UMMA descriptors are then warp-uniform values the compiler keeps in the
-// uniform datapath, instead of per-lane registers that need an R2UR move in front of every tcgen05.mma operand (ncu of the
-// single-lane version: 1.8 M R2UR + 1.3 M IMAD around 0.19 M MMAs; the issuing thread, not the tensor pipe, was the limiter).
+// The producer / issuer warps run their loops with ALL 32 lanes (lane 0 alone issues the TMA loads, elect.sync picks the lane
+// that issues the MMAs and commits): loop counters, stage indices and UMMA descriptors are then warp-uniform values the compiler
+// keeps in the uniform datapath, instead of per-lane registers that need an R2UR move in front of every tcgen05.mma operand (ncu
+// of a lane-0-only version: 1.8 M R2UR + 1.3 M IMAD around 0.19 M MMAs; the issuing thread, not the tensor pipe, was the limiter).
 // EPI: 0 = bf16 out = relu(acc + bias) (the bf16 configuration); fp32-storage configuration, one of three split passes
 // (hi.W_hi, lo.W_hi, hi.W_lo of the bf16 split of an fp32 input, relative error ~2^-16 like gemm_tc_split3):
 // 1 = out_f32 = acc, 2 = out_f32 += acc, 3 = out_f32 = relu(out_f32 + acc + bias).  Every output row is owned by one thread per
 // pass, so the fp32 accumulation across passes needs no atomics.
-template <int CIN, bool UNI, int EPI>
+template <int CIN, int EPI>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv3d_tc_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ CUtensorMap tmW,
                  const float* __restrict__ bias, bf16* __restrict__ out, float* __restrict__ out_f32, int X, int Y)
@@ -87,121 +85,100 @@ conv3d_tc_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant
 
     const bool leader = lane == 0;
     if (warp == 0) {
-        if (UNI || leader) {
-            if (leader) {
-                tc::mbar_arrive_expect_tx(w_bar, TAPS * W_TAP_BYTES);
-                for (int t = 0; t < TAPS; ++t)               // global tap order is (dz,dy,dx); resident order (dz,dy,2-dx)
-                    tc::tma_load_2d(w_base + ((t / 3) * 3 + (2 - t % 3)) * W_TAP_BYTES, &tmW, w_bar, 0, t * COUT);
-            }
-            int s = 0; uint32_t ph = 0;
-            for (int t = t_begin; t < t_end;) {
-                const int yt = t / X, xa = t % X;
-                const int xb = min(X, xa + (t_end - t));
-                const int y0 = yt * TILE_Y;
-                const int p_lo = max(xa - 1, 0), p_hi = min(xb, X - 1);
-                for (int p = p_lo; p <= p_hi; ++p) {
-                    for (int dz = 0; dz < 3; ++dz) {
-                        tc::mbar_wait(empty_bar(s), ph ^ 1);
-                        if (leader) {
-                            tc::mbar_arrive_expect_tx(full_bar(s), A_BYTES);
-                            tc::tma_load_4d(a_base + s * A_BYTES, &tmIn, full_bar(s), 0, dz - 1, y0 - 1, p);
-                        }
-                        if (++s == STAGES) { s = 0; ph ^= 1; }
+        if (leader) {
+            tc::mbar_arrive_expect_tx(w_bar, TAPS * W_TAP_BYTES);
+            for (int t = 0; t < TAPS; ++t)                   // global tap order is (dz,dy,dx); resident order (dz,dy,2-dx)
+                tc::tma_load_2d(w_base + ((t / 3) * 3 + (2 - t % 3)) * W_TAP_BYTES, &tmW, w_bar, 0, t * COUT);
+        }
+        int s = 0; uint32_t ph = 0;
+        for (int t = t_begin; t < t_end;) {
+            const int yt = t / X, xa = t % X;
+            const int xb = min(X, xa + (t_end - t));
+            const int y0 = yt * TILE_Y;
+            const int p_lo = max(xa - 1, 0), p_hi = min(xb, X - 1);
+            for (int p = p_lo; p <= p_hi; ++p) {
+                for (int dz = 0; dz < 3; ++dz) {
+                    tc::mbar_wait(empty_bar(s), ph ^ 1);
+                    if (leader) {
+                        tc::mbar_arrive_expect_tx(full_bar(s), A_BYTES);
+                        tc::tma_load_4d(a_base + s * A_BYTES, &tmIn, full_bar(s), 0, dz - 1, y0 - 1, p);
                     }
+                    if (++s == STAGES) { s = 0; ph ^= 1; }
                 }
-                t += xb - xa;
             }
+            t += xb - xa;
         }
     } else if (warp == 1) {
-        if (UNI || leader) {
-            const uint32_t idesc1 = tc::make_idesc_bf16(BLOCK_M, COUT), idesc2 = tc::make_idesc_bf16(BLOCK_M, 2 * COUT),
-                           idesc3 = tc::make_idesc_bf16(BLOCK_M, 3 * COUT);
-            auto idesc_of = [&](int outputs) { return outputs == 1 ? idesc1 : (outputs == 2 ? idesc2 : idesc3); };
-            const uint64_t da0 = tc::make_smem_desc(a_base, ROW_BYTES), db0 = tc::make_smem_desc(w_base, ROW_BYTES);
-            int s = 0; uint32_t ph = 0;
-            int n_base = 0;
-            if (UNI) tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);     // (a broadcast from lane 0 is a uniform value to ptxas)
-            tc::mbar_wait(w_bar, 0);
-            tc::tc_fence_after();
-            for (int t = t_begin; t < t_end;) {
-                const int xa = t % X;
-                const int xb = min(X, xa + (t_end - t));
-                const int p_lo = max(xa - 1, 0), p_hi = min(xb, X - 1);
-                for (int p = p_lo; p <= p_hi; ++p) {
-                    const int x_lo = max(p - 1, xa), x_hi = min(p + 1, xb - 1);      // outputs this plane feeds
-                    const int cnt = x_hi - x_lo + 1, off = x_lo - (p - 1);            // 1..3 outputs, first weight sub-tile
-                    const int n_lo = n_base + (x_lo - xa), slot_lo = n_lo & (SLOTS - 1);
-                    const int first = min(cnt, SLOTS - slot_lo);                       // outputs before the ring wraps
-                    // outputs whose first plane this is: x = p+1 (and x = 0 on plane 0) -- their slot must be drained + zeroed
-                    for (int x = x_lo; x <= x_hi; ++x) {
-                        if (max(x - 1, 0) != p) continue;
-                        const int n = n_base + (x - xa);
-                        tc::mbar_wait(tempty_bar(n & (SLOTS - 1)), (n / SLOTS) & 1);
-                    }
-                    tc::tc_fence_after();
-                    const uint32_t d0 = tmem_base + slot_lo * COUT;
-                    const uint32_t i_first = idesc_of(first), i_rest = idesc_of(cnt - first);
-                    for (int dz = 0; dz < 3; ++dz) {
-                        tc::mbar_wait(full_bar(s), ph);
-                        tc::tc_fence_after();
-                        if constexpr (UNI) {
-                            // warp-uniform control flow: operands stay in the uniform datapath, elect.sync issues from one lane
-                            const uint32_t desc_hi = (uint32_t)(da0 >> 32);                    // == high word of db0 (same ROW_BYTES)
-                            const uint32_t a_s = (uint32_t)da0 + (uint32_t)((s * A_BYTES) >> 4);
-                            const uint32_t b_z = (uint32_t)db0 + (uint32_t)(((dz * 9 + off) * W_TAP_BYTES) >> 4);
-                            const uint32_t wrap = first < cnt ? 1u : 0u, b_wrap = (uint32_t)((first * W_TAP_BYTES) >> 4);
-                            // one (warp-uniform) branch per STAGE: the 3-output window wraps around the TMEM slot ring for 2 of 8
-                            // positions only, and the second MMA's operand set-up costs as much as the first's
-                            if (!wrap) {
-#pragma unroll
-                                for (int dy = 0; dy < 3; ++dy) {
-#pragma unroll
-                                    for (int k = 0; k < CIN / 16; ++k)
-                                        tc::umma_bf16_acc_elect_lo(d0, a_s + (uint32_t)((dy * DY_BYTES) >> 4) + 2 * k,
-                                                                   b_z + (uint32_t)((dy * 3 * W_TAP_BYTES) >> 4) + 2 * k, desc_hi, i_first);
-                                }
-                            } else {
-#pragma unroll
-                                for (int dy = 0; dy < 3; ++dy) {
-#pragma unroll
-                                    for (int k = 0; k < CIN / 16; ++k) {
-                                        const uint32_t a_lo = a_s + (uint32_t)((dy * DY_BYTES) >> 4) + 2 * k;
-                                        const uint32_t b_lo = b_z + (uint32_t)((dy * 3 * W_TAP_BYTES) >> 4) + 2 * k;
-                                        tc::umma_bf16_acc_elect_lo(d0, a_lo, b_lo, desc_hi, i_first);
-                                        tc::umma_bf16_acc_elect_lo(tmem_base, a_lo, b_lo + b_wrap, desc_hi, i_rest);
-                                    }
-                                }
-                            }
-                            __syncwarp();
-                            tc::umma_commit_elect(empty_bar(s));
-                        } else if (leader) {
-#pragma unroll
-                            for (int dy = 0; dy < 3; ++dy) {
-                                const int t9 = dz * 3 + dy;
-                                const uint64_t da = da0 + (uint64_t)((s * A_BYTES + dy * DY_BYTES) >> 4);
-                                const uint64_t db = db0 + (uint64_t)(((t9 * 3 + off) * W_TAP_BYTES) >> 4);
-#pragma unroll
-                                for (int k = 0; k < CIN / 16; ++k) {
-                                    tc::umma_bf16(d0, da + 2 * k, db + 2 * k, i_first, 1);
-                                    if (first < cnt)
-                                        tc::umma_bf16(tmem_base, da + 2 * k, db + (uint64_t)((first * W_TAP_BYTES) >> 4) + 2 * k, i_rest, 1);
-                                }
-                            }
-                            tc::umma_commit(empty_bar(s));
-                        }
-                        if (UNI) __syncwarp();
-                        if (++s == STAGES) { s = 0; ph ^= 1; }
-                    }
-                    // outputs whose last plane this was: x = p-1 (and x = X-1 on the last plane)
-                    for (int x = x_lo; x <= x_hi; ++x) {
-                        if (min(x + 1, X - 1) != p) continue;
-                        if constexpr (UNI) tc::umma_commit_elect(tfull_bar((n_base + (x - xa)) & (SLOTS - 1)));
-                        else if (leader) tc::umma_commit(tfull_bar((n_base + (x - xa)) & (SLOTS - 1)));
-                    }
+        const uint32_t idesc1 = tc::make_idesc_bf16(BLOCK_M, COUT), idesc2 = tc::make_idesc_bf16(BLOCK_M, 2 * COUT),
+                       idesc3 = tc::make_idesc_bf16(BLOCK_M, 3 * COUT);
+        auto idesc_of = [&](int outputs) { return outputs == 1 ? idesc1 : (outputs == 2 ? idesc2 : idesc3); };
+        const uint64_t da0 = tc::make_smem_desc(a_base, ROW_BYTES), db0 = tc::make_smem_desc(w_base, ROW_BYTES);
+        int s = 0; uint32_t ph = 0;
+        int n_base = 0;
+        tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);     // (a broadcast from lane 0 is a uniform value to ptxas)
+        tc::mbar_wait(w_bar, 0);
+        tc::tc_fence_after();
+        for (int t = t_begin; t < t_end;) {
+            const int xa = t % X;
+            const int xb = min(X, xa + (t_end - t));
+            const int p_lo = max(xa - 1, 0), p_hi = min(xb, X - 1);
+            for (int p = p_lo; p <= p_hi; ++p) {
+                const int x_lo = max(p - 1, xa), x_hi = min(p + 1, xb - 1);      // outputs this plane feeds
+                const int cnt = x_hi - x_lo + 1, off = x_lo - (p - 1);            // 1..3 outputs, first weight sub-tile
+                const int n_lo = n_base + (x_lo - xa), slot_lo = n_lo & (SLOTS - 1);
+                const int first = min(cnt, SLOTS - slot_lo);                       // outputs before the ring wraps
+                // outputs whose first plane this is: x = p+1 (and x = 0 on plane 0) -- their slot must be drained + zeroed
+                for (int x = x_lo; x <= x_hi; ++x) {
+                    if (max(x - 1, 0) != p) continue;
+                    const int n = n_base + (x - xa);
+                    tc::mbar_wait(tempty_bar(n & (SLOTS - 1)), (n / SLOTS) & 1);
                 }
-                n_base += xb - xa;
-                t += xb - xa;
+                tc::tc_fence_after();
+                const uint32_t d0 = tmem_base + slot_lo * COUT;
+                const uint32_t i_first = idesc_of(first), i_rest = idesc_of(cnt - first);
+                for (int dz = 0; dz < 3; ++dz) {
+                    tc::mbar_wait(full_bar(s), ph);
+                    tc::tc_fence_after();
+                    // warp-uniform control flow: operands stay in the uniform datapath, elect.sync issues from one lane
+                    const uint32_t desc_hi = (uint32_t)(da0 >> 32);                    // == high word of db0 (same ROW_BYTES)
+                    const uint32_t a_s = (uint32_t)da0 + (uint32_t)((s * A_BYTES) >> 4);
+                    const uint32_t b_z = (uint32_t)db0 + (uint32_t)(((dz * 9 + off) * W_TAP_BYTES) >> 4);
+                    const uint32_t wrap = first < cnt ? 1u : 0u, b_wrap = (uint32_t)((first * W_TAP_BYTES) >> 4);
+                    // one (warp-uniform) branch per STAGE: the 3-output window wraps around the TMEM slot ring for 2 of 8
+                    // positions only, and the second MMA's operand set-up costs as much as the first's
+                    if (!wrap) {
+#pragma unroll
+                        for (int dy = 0; dy < 3; ++dy) {
+#pragma unroll
+                            for (int k = 0; k < CIN / 16; ++k)
+                                tc::umma_bf16_acc_elect_lo(d0, a_s + (uint32_t)((dy * DY_BYTES) >> 4) + 2 * k,
+                                                           b_z + (uint32_t)((dy * 3 * W_TAP_BYTES) >> 4) + 2 * k, desc_hi, i_first);
+                        }
+                    } else {
+#pragma unroll
+                        for (int dy = 0; dy < 3; ++dy) {
+#pragma unroll
+                            for (int k = 0; k < CIN / 16; ++k) {
+                                const uint32_t a_lo = a_s + (uint32_t)((dy * DY_BYTES) >> 4) + 2 * k;
+                                const uint32_t b_lo = b_z + (uint32_t)((dy * 3 * W_TAP_BYTES) >> 4) + 2 * k;
+                                tc::umma_bf16_acc_elect_lo(d0, a_lo, b_lo, desc_hi, i_first);
+                                tc::umma_bf16_acc_elect_lo(tmem_base, a_lo, b_lo + b_wrap, desc_hi, i_rest);
+                            }
+                        }
+                    }
+                    __syncwarp();
+                    tc::umma_commit_elect(empty_bar(s));
+                    __syncwarp();
+                    if (++s == STAGES) { s = 0; ph ^= 1; }
+                }
+                // outputs whose last plane this was: x = p-1 (and x = X-1 on the last plane)
+                for (int x = x_lo; x <= x_hi; ++x) {
+                    if (min(x + 1, X - 1) != p) continue;
+                    tc::umma_commit_elect(tfull_bar((n_base + (x - xa)) & (SLOTS - 1)));
+                }
             }
+            n_base += xb - xa;
+            t += xb - xa;
         }
     } else {
         const int quarter = warp & 3;
@@ -299,19 +276,9 @@ int launch_conv3d_tc_impl(const bf16* in, int in_pitch, const bf16* w_tap_major,
     const int num_sms = sm_count_current_device();
     const int tiles = X * ((Y + TILE_Y - 1) / TILE_Y);
     const int grid = tiles < num_sms ? tiles : num_sms;
-    static const bool uni = getenv("OCC_CONV_SINGLE_LANE") == nullptr;      // OCC_CONV_SINGLE_LANE=1: the lane-0-only loops (EPI 0 only)
-#define OCC_CONV_LAUNCH(C, U)                                                                                          \
-    do {                                                                                                               \
-        OCC_CUDA(cudaFuncSetAttribute(conv3d_tc_kernel<C, U, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        conv3d_tc_kernel<C, U, EPI><<<grid, NUM_THREADS, smem, stream>>>(tmIn, tmW, bias, out, out_f32, X, Y);         \
-    } while (0)
-    if constexpr (EPI == 0) {
-        if (Cin == 16) { if (uni) OCC_CONV_LAUNCH(16, true); else OCC_CONV_LAUNCH(16, false); }
-        else           { if (uni) OCC_CONV_LAUNCH(32, true); else OCC_CONV_LAUNCH(32, false); }
-    } else {
-        if (Cin == 16) OCC_CONV_LAUNCH(16, true); else OCC_CONV_LAUNCH(32, true);
-    }
-#undef OCC_CONV_LAUNCH
+    const auto kernel = Cin == 16 ? conv3d_tc_kernel<16, EPI> : conv3d_tc_kernel<32, EPI>;
+    OCC_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    kernel<<<grid, NUM_THREADS, smem, stream>>>(tmIn, tmW, bias, out, out_f32, X, Y);
     OCC_CUDA(cudaGetLastError());
     return 0;
 }

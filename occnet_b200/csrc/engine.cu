@@ -65,9 +65,6 @@ struct occb200_engine {
     LevelGeom lg;
     ScaParams sp;
     bool cameras_set = false, finalized = false, taps = false;
-    bool value_head_major = false;      // SCA value maps as [layer][head][token][32] (pair-fetch gather) instead of [layer][token][256]
-    bool gemm_chain = false;            // OCC_GEMM_CHAIN=1 at finalize: chained dense layers (gemm_chain.cu)
-    DevBuf sca_sched;                   // scheduler words of the SM-tiled gather kernel (zeroed by every launch)
     DevBuf rot_map;                     // occb200_engine_set_prev_rotation: source row of every BEV cell (int32, -1 = outside)
     bool rot_set = false;
     int feats_bf16 = 0;                 // occb200_engine_set_input_dtype: feature levels arrive as bf16 instead of fp32
@@ -303,8 +300,7 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
     // the gather kernel; |offset| is a few pixels, so fp16's 11-bit mantissa keeps locations to < 0.01 px), fp32 otherwise
     const int nq_tsa = 2 * 8 * c.tsa_points * 3;   // offsets (x,y) + logits
     const int nq_sca = 8 * c.num_levels * c.sca_points * 3;
-    static const bool q_f32_env = getenv("OCC_QPROJ_F32") != nullptr;
-    const bool q_half = sizeof(T) == 2 && c.use_tensor_cores && !q_f32_env && e->layers[0].tsa_q_wh.p != nullptr &&
+    const bool q_half = sizeof(T) == 2 && c.use_tensor_cores && e->layers[0].tsa_q_wh.p != nullptr &&
                         e->layers[0].sca_q_wh.p != nullptr && gemm_tc_supported(Nq, nq_tsa, 2 * C, C) &&
                         gemm_tc_supported(Nq, nq_sca, C, C);
     void* qproj = e->qproj.p;
@@ -317,23 +313,13 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
         e->launches++;
         ProfScope ps(e, st, CAT_GEMM);
         if (gemm_tc_blocked256((const bf16*)tokens, e->sca_v_all_wh.as<bf16>(), e->sca_v_all_b.as<float>(),
-                               e->sca_value_all.as<bf16>(), ncam * Nv, c.num_layers * C, C, st, e->value_head_major)) return 2;
+                               e->sca_value_all.as<bf16>(), ncam * Nv, c.num_layers * C, C, st)) return 2;
     }
-    // Chained dense layers (gemm_chain.cu, OCC_GEMM_CHAIN=1): [TSA output_proj+LN -> SCA sampling projection] and [SCA
-    // output_proj+LN -> FFN1 -> FFN2+LN -> next layer's TSA value / sampling projections] as ONE persistent launch each: 30 launches
-    // per frame instead of 52 (13 dense-layer launches), bit-identical outputs -- and MEASURED 3 % SLOWER per frame (2.94 vs 2.86 ms,
-    // r2 call 11): every (op, n-block) switch inside the kernel re-pays the 128 KB weight load that a fresh launch pays, and the
-    // per-tile epilogues were already the bound.  Off by default.
-    const bool use_chain = sizeof(T) == 2 && fuse_ln && q_half && e->gemm_chain && mode == MODE_FRAME && !e->value_head_major;
-    static const bool tsa_merge_env0 = getenv("OCC_TSA_MERGE") == nullptr || atoi(getenv("OCC_TSA_MERGE")) != 0;
-    const bool tsa_merge_ok = tsa_merge_env0;
-    bool tsa_inputs_done = false;           // this layer's TSA value / sampling projections were written by the previous chain
     for (int l = 0; l < c.num_layers; ++l) {
         LayerW& w = e->layers[l];
         // self mode (prev_bev = None): W1 q + W2 (q + pos) = (W1 + W2) q + W2 pos -- the second operand is the CONSTANT
         // bf16 pos, so no layer has to write (and the FFN LayerNorm epilogue has to read pos for) a bf16 copy of q + pos
         const bool fold_pos = fuse_ln && !has_prev && w.tsa_q_wh_fold.p != nullptr && w.tsa_q_const.p != nullptr && q_half;
-        bool sca_q_done = false;                                // the SCA sampling projection was the tail of the TSA chain
         // ---- temporal self-attention (temporal_self_attention.py:177-272)
         if (l == 0 && l0_fold) {
             // precomputed at finalize: residual stream := constant T32 buffer, SCA projection operand := constant bf16 copy
@@ -344,27 +330,15 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
         } else {
         T* v_cur = e->tsa_value.as<T>();
         T* v_prev = v_cur;
-        // head-major value maps + pair-fetch gather on the fused tensor-core path (same layout trick as the SCA values)
-        static const bool tsa_rowmajor_env = getenv("OCC_TSA_ROWMAJOR") != nullptr;
-        const bool tsa_hm = fuse_ln && e->value_head_major && q_half && !tsa_rowmajor_env;
         auto value_gemm = [&](const T* a, T* dst) -> int {
-            if (tsa_hm) {
-                e->launches++;
-                ProfScope ps(e, st, CAT_GEMM);
-                return gemm_tc_heads256(reinterpret_cast<const bf16*>(a), w.tsa_v_wh.as<bf16>(), w.tsa_v_b.as<float>(),
-                                        reinterpret_cast<bf16*>(dst), Nq, C, st);
-            }
             return gemm<T, T>(e, a, nullptr, 0, w.tsa_v_w.as<float>(), w.tsa_v_wh.p, w.tsa_v_b.as<float>(), nullptr, dst, Nq, C, C,
                               ACT_NONE, st);
         };
         // value_proj of every queue entry + the sampling projection are independent GEMMs over [Nq,256] operands: ONE launch on
-        // disjoint CTA ranges (OCC_TSA_MERGE=0: one launch each)
-        static const bool tsa_merge_env = getenv("OCC_TSA_MERGE") == nullptr || atoi(getenv("OCC_TSA_MERGE")) != 0;
-        const bool tsa_merge = sizeof(T) == 2 && fuse_ln && q_half && !tsa_hm && tsa_merge_env && w.tsa_v_wh.p != nullptr;
+        // disjoint CTA ranges
+        const bool tsa_merge = sizeof(T) == 2 && fuse_ln && q_half && w.tsa_v_wh.p != nullptr;
         if (has_prev) v_prev = e->tsa_value_prev.as<T>();
-        if (tsa_inputs_done) {
-            tsa_inputs_done = false;                             // (written by the tail of the previous layer's chain)
-        } else if (tsa_merge) {
+        if (tsa_merge) {
             if constexpr (sizeof(T) == 2) {
                 const bf16* Av[2] = {reinterpret_cast<const bf16*>(has_prev ? q0_t : q_in), e->prev_t.as<bf16>()};
                 bf16* Cv[2] = {reinterpret_cast<bf16*>(v_cur), reinterpret_cast<bf16*>(v_prev)};
@@ -399,29 +373,9 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
         }   // (tsa_merge)
         {
             ProfScope ps(e, st, CAT_TSA);
-            if (tsa_hm) {
-                if (launch_tsa_pair(reinterpret_cast<const bf16*>(v_prev), reinterpret_cast<const bf16*>(v_cur), qproj, q_half,
-                                    c.bev_h, c.bev_w, reinterpret_cast<bf16*>(attn_out), st)) return 2;
-            } else if (launch_tsa_fused<T>(v_prev, v_cur, qproj, q_half, c.bev_h, c.bev_w, attn_out, st)) return 2;
+            if (launch_tsa_fused<T>(v_prev, v_cur, qproj, q_half, c.bev_h, c.bev_w, attn_out, st)) return 2;
         }
         e->launches++;
-        if (use_chain) {
-            if constexpr (sizeof(T) == 2) {
-                GemmChainOp ops[2];
-                memset(ops, 0, sizeof(ops));
-                ops[0].A = reinterpret_cast<const bf16*>(attn_out); ops[0].K1 = C; ops[0].W = w.tsa_o_wh.as<bf16>(); ops[0].N = C; ops[0].K = C;
-                ops[0].bias = w.tsa_o_b.as<float>(); ops[0].ln = 1; ops[0].residual = q_f32; ops[0].gamma = w.ln_g[0].as<float>();
-                ops[0].beta = w.ln_b[0].as<float>(); ops[0].y_f32 = x_f32; ops[0].y_bf16 = reinterpret_cast<bf16*>(q_t);
-                ops[1].A = reinterpret_cast<const bf16*>(q_t); ops[1].K1 = C; ops[1].W = w.sca_q_wh.as<bf16>(); ops[1].N = nq_sca; ops[1].K = C;
-                ops[1].bias = w.sca_q_b.as<float>(); ops[1].dep = 1; ops[1].C = qproj; ops[1].out_half = 1; ops[1].act = ACT_NONE;
-                e->launches++;
-                ProfScope ps(e, st, CAT_GEMM);
-                if (gemm_chain_launch(ops, 2, Nq, st)) return 2;
-            }
-            advance();
-            q_in = q_t; q_pos_in = q_pos_t;
-            sca_q_done = true;
-        } else
         if (fuse_ln) {
             float* y32 = mode == MODE_L0_TSA_ONLY ? e->l0_x_f32.as<float>() : x_f32;
             bf16* y16 = mode == MODE_L0_TSA_ONLY ? e->l0_q_t.as<bf16>() : (bf16*)q_t;
@@ -445,9 +399,7 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
         }
         }   // (layer-0 TSA fold)
         // ---- spatial cross-attention (spatial_cross_attention.py:128-175, :334-393)
-        if (sca_q_done) {
-            q_t_in = q_t;
-        } else {
+        {
             const int rc = q_half ? gemm<T, __half>(e, q_t_in, nullptr, 0, w.sca_q_w.as<float>(), w.sca_q_wh.p, w.sca_q_b.as<float>(),
                                                     nullptr, (__half*)qproj, Nq, nq_sca, C, ACT_NONE, st)
                                   : gemm<T, float>(e, q_t_in, nullptr, 0, w.sca_q_w.as<float>(), w.sca_q_wh.p, w.sca_q_b.as<float>(),
@@ -457,55 +409,14 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
         }
         const T* sca_val = e->sca_value.as<T>();
         if (hoist_v) {
-            static const size_t hack2 = (getenv("OCC_PAIR_HACK") && atoi(getenv("OCC_PAIR_HACK")) == 2) ? 2 : 1;
-            sca_val = reinterpret_cast<const T*>(e->sca_value_all.as<bf16>() + (size_t)l * ncam * Nv * C * hack2);
+            sca_val = reinterpret_cast<const T*>(e->sca_value_all.as<bf16>() + (size_t)l * ncam * Nv * C);
         } else if (gemm<T, T>(e, tokens, nullptr, 0, w.sca_v_w.as<float>(), w.sca_v_wh.p, w.sca_v_b.as<float>(), nullptr,
                               e->sca_value.as<T>(), ncam * Nv, C, C, ACT_NONE, st)) return 2;
         {
             ProfScope ps(e, st, CAT_SCA);
-            if (hoist_v && e->value_head_major) {
-                if (launch_sca_pair(reinterpret_cast<const bf16*>(sca_val), qproj, q_half, e->sp, e->lg, Nv,
-                                    reinterpret_cast<bf16*>(attn_out), e->hits.as<uint8_t>(), st)) return 2;
-            } else if (launch_sca_fused<T>(sca_val, qproj, q_half, e->sp, e->lg, Nv, attn_out, e->hits.as<uint8_t>(), st,
-                                           e->sca_sched.as<unsigned>())) return 2;
+            if (launch_sca_fused<T>(sca_val, qproj, q_half, e->sp, e->lg, Nv, attn_out, e->hits.as<uint8_t>(), st)) return 2;
         }
         e->launches++;
-        if (use_chain) {
-            if constexpr (sizeof(T) == 2) {
-                GemmChainOp ops[5];
-                memset(ops, 0, sizeof(ops));
-                int n = 0;
-                const bool need_qpos = !fold_pos;
-                ops[n].A = reinterpret_cast<const bf16*>(attn_out); ops[n].K1 = C; ops[n].W = w.sca_o_wh.as<bf16>(); ops[n].N = C; ops[n].K = C;
-                ops[n].bias = w.sca_o_b.as<float>(); ops[n].ln = 1; ops[n].residual = q_f32; ops[n].gamma = w.ln_g[1].as<float>();
-                ops[n].beta = w.ln_b[1].as<float>(); ops[n].y_f32 = x_f32; ops[n].y_bf16 = reinterpret_cast<bf16*>(q_t);
-                ++n; advance();
-                ops[n].A = reinterpret_cast<const bf16*>(q_t); ops[n].K1 = C; ops[n].W = w.ffn1_wh.as<bf16>(); ops[n].N = c.ffn_dim; ops[n].K = C;
-                ops[n].bias = w.ffn1_b.as<float>(); ops[n].dep = 1; ops[n].C = e->ffn_h.p; ops[n].act = ACT_RELU;
-                ++n;
-                ops[n].A = e->ffn_h.as<bf16>(); ops[n].K1 = c.ffn_dim; ops[n].W = w.ffn2_wh.as<bf16>(); ops[n].N = C; ops[n].K = c.ffn_dim;
-                ops[n].bias = w.ffn2_b.as<float>(); ops[n].dep = 1; ops[n].ln = 1; ops[n].residual = q_f32; ops[n].gamma = w.ln_g[2].as<float>();
-                ops[n].beta = w.ln_b[2].as<float>(); ops[n].y_f32 = x_f32; ops[n].y_bf16 = reinterpret_cast<bf16*>(q_t);
-                if (need_qpos) { ops[n].pos = e->pos_t32.as<float>(); ops[n].y_pos_bf16 = reinterpret_cast<bf16*>(q_pos_t); }
-                ++n; advance();
-                // next layer's TSA inputs (self mode): value_proj and the folded sampling projection read the LayerNorm output
-                if (l + 1 < c.num_layers && !has_prev && tsa_merge_ok) {
-                    LayerW& wn = e->layers[l + 1];
-                    if (wn.tsa_q_wh_fold.p && wn.tsa_q_const_t32.p && wn.tsa_v_wh.p) {
-                        ops[n].A = reinterpret_cast<const bf16*>(q_t); ops[n].K1 = C; ops[n].W = wn.tsa_v_wh.as<bf16>(); ops[n].N = C; ops[n].K = C;
-                        ops[n].bias = wn.tsa_v_b.as<float>(); ops[n].dep = 1; ops[n].C = e->tsa_value.p;
-                        ++n;
-                        ops[n].A = reinterpret_cast<const bf16*>(q_t); ops[n].K1 = C; ops[n].W = wn.tsa_q_wh_fold.as<bf16>(); ops[n].N = nq_tsa; ops[n].K = C;
-                        ops[n].dep = 1; ops[n].C = qproj; ops[n].out_half = 1; ops[n].res_t32 = wn.tsa_q_const_t32.as<float>();
-                        ++n;
-                        tsa_inputs_done = true;
-                    }
-                }
-                e->launches++;
-                ProfScope ps(e, st, CAT_GEMM);
-                if (gemm_chain_launch(ops, n, Nq, st)) return 2;
-            }
-        } else
         if (fuse_ln) {
             if (gemm_ln_fused(e, (const bf16*)attn_out, w.sca_o_wh.p, w.sca_o_b.as<float>(), q_f32, w.ln_g[1].as<float>(),
                               w.ln_b[1].as<float>(), nullptr, x_f32, (bf16*)q_t, nullptr, Nq, C, st)) return 2;
@@ -524,9 +435,6 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
             e->launches++;
         }
         // ---- FFN (mmcv FFN: x + W2 relu(W1 x))
-        if (use_chain) {
-            // (FFN1, FFN2 + LayerNorm were ops 1-2 of the chain above)
-        } else {
         if (gemm<T, T>(e, q_t, nullptr, 0, w.ffn1_w.as<float>(), w.ffn1_wh.p, w.ffn1_b.as<float>(), nullptr,
                        e->ffn_h.as<T>(), Nq, c.ffn_dim, C, ACT_RELU, st)) return 2;
         if (fuse_ln) {
@@ -546,7 +454,6 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
             }
             e->launches++;
         }
-        }   // (!use_chain)
         if (e->taps)
             OCC_CUDA(cudaMemcpyAsync(e->tap_layer.as<float>() + (size_t)l * Nq * C, q_f32, (size_t)Nq * C * 4,
                                      cudaMemcpyDeviceToDevice, st));
@@ -571,9 +478,8 @@ int forward_impl(occb200_engine* e, const float* const* feats, const float* prev
         } else if (launch_bev_to_voxel<T>(q_f32, c.bev_h, c.bev_w, Z, mid, e->vox0.as<T>(), st)) return 2;
     }
     const bool conv_tc = sizeof(T) == 2 && c.use_tensor_cores && e->conv_wh[0].p && e->conv_wh[1].p && Z == 16;
-    // fp32 storage + tensor cores: both convolutions as three bf16-split passes accumulated in fp32 (OCC_CONV_F32_SIMT=1: CUDA cores)
-    static const bool conv_simt_env = getenv("OCC_CONV_F32_SIMT") != nullptr;
-    const bool conv_split = sizeof(T) == 4 && c.use_tensor_cores && !conv_simt_env && e->conv_wh_hi[0].p && e->conv_wh_lo[1].p &&
+    // fp32 storage + tensor cores: both convolutions as three bf16-split passes accumulated in fp32
+    const bool conv_split = sizeof(T) == 4 && c.use_tensor_cores && e->conv_wh_hi[0].p && e->conv_wh_lo[1].p &&
                             e->vox_split.p && Z == 16 && (mid == 16 || mid == 32) && c.out_dim == 32;
     if (conv_split) {
         const int64_t nv = (int64_t)X * Y * Z;
@@ -699,7 +605,7 @@ void occb200_engine_destroy(occb200_engine* e)
                          &w.tsa_q_wh_fold, &w.tsa_q_const, &w.tsa_q_const_t32};
         for (DevBuf* b : all) b->release();
     }
-    DevBuf* all[] = {&e->sca_sched, &e->rot_map, &e->split_ws, &e->tokens_split, &e->l0_x_f32, &e->l0_q_t, &e->pos_bf, &e->qc_f32, &e->qc_t, &e->qc_pos_t, &e->bev_queries, &e->pos, &e->pos_t32, &e->cams_embeds, &e->level_embeds, &e->conv_w[0], &e->conv_w[1],
+    DevBuf* all[] = {&e->rot_map, &e->split_ws, &e->tokens_split, &e->l0_x_f32, &e->l0_q_t, &e->pos_bf, &e->qc_f32, &e->qc_t, &e->qc_pos_t, &e->bev_queries, &e->pos, &e->pos_t32, &e->cams_embeds, &e->level_embeds, &e->conv_w[0], &e->conv_w[1],
                      &e->conv_b[0], &e->conv_b[1], &e->conv_wh[0], &e->conv_wh[1], &e->conv_wh_hi[0], &e->conv_wh_hi[1], &e->conv_wh_lo[0],
                      &e->conv_wh_lo[1], &e->vox_split, &e->sca_v_all_wh, &e->sca_v_all_b, &e->sca_value_all, &e->hw1, &e->hb1, &e->hw2, &e->hb2,
                      &e->fw1, &e->fb1, &e->fw2, &e->fb2, &e->head_w1h, &e->head_w2h, &e->head_b1c, &e->head_b2c, &e->tokens, &e->sca_value, &e->q_f32, &e->q_t,
@@ -863,12 +769,8 @@ int occb200_engine_finalize(occb200_engine* e)
             B.insert(B.end(), b->begin(), b->end());
         }
         if (upload_bf16(e->sca_v_all_wh, W.data(), W.size()) || upload(e->sca_v_all_b, B.data(), B.size())) return 2;
-        const size_t hack2 = (getenv("OCC_PAIR_HACK") && atoi(getenv("OCC_PAIR_HACK")) == 2) ? 2 : 1;   // timing experiment: 128-byte token pitch
-        if (e->sca_value_all.alloc((size_t)c.num_layers * c.num_cams * e->Nv * C * 2 * hack2 + 256)) return 2;   // (+ one pair over-read)
+        if (e->sca_value_all.alloc((size_t)c.num_layers * c.num_cams * e->Nv * C * 2)) return 2;
         OCC_CUDA(cudaMemset(e->sca_value_all.p, 0, e->sca_value_all.bytes));
-        // OCC_VALUE_HEADMAJOR=1: head-major value maps + pair-fetch gathers (sca_pair / tsa_pair).  MEASURED SLOWER than the
-        // row-major layout + sca_pipe / tsa_fused (SCA 1.63 vs 1.32 ms, TSA 0.31 vs 0.23 ms per frame): kept as an experiment
-        e->value_head_major = getenv("OCC_VALUE_HEADMAJOR") != nullptr;
     }
     // decoder: fold BatchNorm3d (eval) into the conv weights; torch layout [Cout][Cin][kz][ky][kx] -> [tap][Cin][Cout]
     for (int i = 0; i < 2; ++i) {
@@ -949,7 +851,7 @@ int occb200_engine_finalize(occb200_engine* e)
         e->tsa_value_prev.alloc((size_t)Nq * C * es) || e->qproj.alloc((size_t)Nq * maxq * 4) ||
         e->attn_out.alloc((size_t)Nq * C * es) || e->x_f32.alloc(nq_pad * C * 4) ||
         e->ffn_h.alloc((size_t)Nq * F * es) || e->vox0.alloc(nvox * mid * es) || e->vox1.alloc(nvox * od * es) ||
-        e->vox2.alloc(nvox * od * es) || e->hits.alloc(Nq) || e->sca_sched.alloc(SCA_SCHED_WORDS * sizeof(unsigned))) return 2;
+        e->vox2.alloc(nvox * od * es) || e->hits.alloc(Nq)) return 2;
     OCC_CUDA(cudaMemset(e->q_f32.p, 0, nq_pad * C * 4));
     OCC_CUDA(cudaMemset(e->x_f32.p, 0, nq_pad * C * 4));
     if (tc32) {
@@ -959,7 +861,6 @@ int occb200_engine_finalize(occb200_engine* e)
     }
     e->host_params.clear();
     e->l0_ready = false;
-    e->gemm_chain = getenv("OCC_GEMM_CHAIN") != nullptr && atoi(getenv("OCC_GEMM_CHAIN")) != 0;
     if (tc && e->qc_f32.p != nullptr && getenv("OCC_NO_L0_FOLD") == nullptr) {
         // Layer 0's TemporalSelfAttention (value_proj, query projection over [bev_queries | pos], gather, output_proj) and
         // its LayerNorm depend on parameters only when prev_bev is None: run the frame path's own kernels once, here.

@@ -98,8 +98,7 @@ struct GemmProb {
     const float* res_t32;                                     // optional fp32 epilogue constant [M,N] in the T32 block layout
                                                               // (TMA-store path: the row-per-thread read is then coalesced)
     long long ldc, nblk_stride;
-    int c_tma /* 0: none, 1: [M,N] row-major, 2: n-blocks as separate [M,BN] matrices,
-                 3: head-major value maps [n-block][column/32][M][32] (one 64-byte row per (head, token)) */;
+    int c_tma /* 0: none, 1: [M,N] row-major, 2: n-blocks as separate [M,BN] matrices */;
     int stg_bytes, M, N, BN, nk, nk1, act, w_resident, stages;
     int out_half;                                             // 16-bit outputs as fp16 instead of bf16 (runtime, per problem)
     int cta_begin, cta_count;
@@ -438,9 +437,8 @@ gemm_tc_kernel(const __grid_constant__ GemmProbs probs, LnArgs ln, long long* __
                     tc::fence_proxy_async_smem();
                     __syncwarp();
                     if (lane == 0) {
-                        if (c_tma == 3)      tc::tma_store_4d(&tmC, stg, 0, row0, c0 >> 5, n_blk);
-                        else if (c_tma == 2) tc::tma_store_3d(&tmC, stg, c0, row0, n_blk);
-                        else                 tc::tma_store_3d(&tmC, stg, col, row0, 0);
+                        if (c_tma == 2) tc::tma_store_3d(&tmC, stg, c0, row0, n_blk);
+                        else            tc::tma_store_3d(&tmC, stg, col, row0, 0);
                         tc::tma_store_commit();
                     }
                 }
@@ -544,7 +542,7 @@ struct MapKey {
 
 }  // namespace
 
-// row-major bf16 [rows, inner] with a row pitch of `ld` elements (0 = dense)  (also used by gemm_chain.cu)
+// row-major bf16 [rows, inner] with a row pitch of `ld` elements (0 = dense)
 int cached_map_2d(const void* base, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows, CUtensorMap* out,
                   uint64_t ld)
 {
@@ -588,36 +586,15 @@ int cached_map_out(const void* base, uint64_t cols, uint64_t rows, uint64_t bloc
 
 namespace {
 
-// head-major output map for c_tma == 3: dims {32 channels, rows, heads = BN/32, n-blocks}, box {32, 32, 1, 1}
-int cached_map_out_heads(const void* base, uint64_t rows, uint64_t heads, uint64_t blocks, CUtensorMap* out)
-{
-    static std::map<std::tuple<const void*, uint64_t, uint64_t, uint64_t>, CUtensorMap> cache;
-    static std::mutex mu;
-    std::lock_guard<std::mutex> g(mu);
-    const auto k = std::make_tuple(base, rows, heads, blocks);
-    auto it = cache.find(k);
-    if (it == cache.end()) {
-        CUtensorMap m;
-        const uint64_t dims[4] = {32, rows, heads, blocks}, strides[3] = {64, rows * 64, heads * rows * 64};
-        const uint32_t box[4] = {32, 32, 1, 1};
-        if (make_tensor_map_bf16(&m, base, 4, dims, strides, box, 64)) return 1;
-        if (cache.size() > 4096) cache.clear();
-        it = cache.emplace(k, m).first;
-    }
-    *out = it->second;
-    return 0;
-}
-
 // Fills one problem (tensor maps, plan, CTA share).  ctas = number of CTAs this problem may use (0: all SMs).
 template <typename TC, bool LN>
 int build_prob(GemmProb& P, int& smem, const bf16* A, const bf16* A2, int K1, const bf16* W, const float* bias, const float* residual,
-               TC* C, int M, int N, int K, int act, bool blocked_out, int lda, int lda2, bool head_major, int ctas, int cta_begin)
+               TC* C, int M, int N, int K, int act, bool blocked_out, int lda, int lda2, int ctas, int cta_begin)
 {
     if (A2 == nullptr) K1 = K;
-    // 16-bit outputs without a residual leave through TMA stores of [32 rows x 32 columns] (OCC_GEMM_NO_TMA_STORE=1:
-    // per-lane stores): a 2 KB staging block per warp instead of 4 KB, which buys one or two more operand stages
-    static const bool no_tma_store = getenv("OCC_GEMM_NO_TMA_STORE") != nullptr;
-    const bool use_tma_store = !LN && sizeof(TC) == 2 && residual == nullptr && C != nullptr && !no_tma_store;
+    // 16-bit outputs without a residual leave through TMA stores of [32 rows x 32 columns]: a 2 KB staging block per warp
+    // instead of 4 KB, which buys one or two more operand stages
+    const bool use_tma_store = !LN && sizeof(TC) == 2 && residual == nullptr && C != nullptr;
     const int stg_bytes = use_tma_store ? 2048 : 4096;
     const Plan p = make_plan(N, K, LN, stg_bytes);
     OCC_CHECK(p.BN > 0 && p.stages >= 2 && K % 64 == 0 && K1 % 64 == 0 && M > 0, "gemm_tc: unsupported shape");
@@ -629,10 +606,7 @@ int build_prob(GemmProb& P, int& smem, const bf16* A, const bf16* A2, int K1, co
     P.c_tma = 0;
     if (use_tma_store) {
         const uint32_t box_cols = 32u;
-        if (head_major) {
-            if (cached_map_out_heads(C, (uint64_t)M, (uint64_t)(p.BN / 32), (uint64_t)(N / p.BN), &P.tmC)) return 1;
-            P.c_tma = 3;
-        } else if (blocked_out) {
+        if (blocked_out) {
             if (cached_map_out(C, (uint64_t)p.BN, (uint64_t)M, (uint64_t)(N / p.BN), box_cols, &P.tmC)) return 1;
             P.c_tma = 2;
         } else {
@@ -702,13 +676,12 @@ int launch_probs(const GemmProbs& probs, int smem, LnArgs ln, cudaStream_t strea
 
 template <typename TC, bool LN>
 int launch(const bf16* A, const bf16* A2, int K1, const bf16* W, const float* bias, const float* residual, TC* C,
-           LnArgs ln, int M, int N, int K, int act, cudaStream_t stream, bool blocked_out = false, int lda = 0, int lda2 = 0,
-           bool head_major = false)
+           LnArgs ln, int M, int N, int K, int act, cudaStream_t stream, bool blocked_out = false, int lda = 0, int lda2 = 0)
 {
     GemmProbs probs;
     probs.n = 1;
     int smem = 0;
-    if (build_prob<TC, LN>(probs.p[0], smem, A, A2, K1, W, bias, residual, C, M, N, K, act, blocked_out, lda, lda2, head_major, 0, 0))
+    if (build_prob<TC, LN>(probs.p[0], smem, A, A2, K1, W, bias, residual, C, M, N, K, act, blocked_out, lda, lda2, 0, 0))
         return 1;
     return launch_probs<TC, LN>(probs, smem, ln, stream);
 }
@@ -728,12 +701,6 @@ int gemm_tc(const bf16* A, const bf16* A2, int K1, const bf16* W, const float* b
     return launch<TC, false>(A, A2, K1, W, bias, residual, C, LnArgs{}, M, N, K, act, stream);
 }
 
-// C = A.W^T + bias, N = 256, written head-major: [8 heads][M][32] bf16 (TMA-store epilogue) -- TSA value maps
-int gemm_tc_heads256(const bf16* A, const bf16* W, const float* bias, bf16* C, int M, int K, cudaStream_t stream)
-{
-    return launch<bf16, false>(A, nullptr, 0, W, bias, nullptr, C, LnArgs{}, M, 256, K, ACT_NONE, stream, false, 0, 0, true);
-}
-
 // fp32-grade GEMM on the tensor cores: S = [hi | lo] (bf16 split of an fp32 operand, row pitch 2*Ks), W3 = [W_hi | W_hi | W_lo]
 // (N x 3*Ks).  C = hi.W_hi + lo.W_hi + hi.W_lo  (the lo.lo term, 2^-16 relative, is dropped) as ONE GEMM with K' = 3*Ks whose
 // A operand is the concatenation [S (2*Ks columns) | first Ks columns of S again] -- two tensor maps over the same buffer.
@@ -743,14 +710,11 @@ int gemm_tc_split3(const bf16* S, int Ks, const bf16* W3, const float* bias, con
     return launch<float, false>(S, S, 2 * Ks, W3, bias, residual, C, LnArgs{}, M, N, 3 * Ks, act, stream, false, 2 * Ks, 2 * Ks);
 }
 
-int gemm_tc_blocked256(const bf16* A, const bf16* W, const float* bias, bf16* C, int M, int N, int K, cudaStream_t stream,
-                       bool head_major)
+int gemm_tc_blocked256(const bf16* A, const bf16* W, const float* bias, bf16* C, int M, int N, int K, cudaStream_t stream)
 {
     const Plan p = make_plan(N, K, false);
     OCC_CHECK(p.BN == 256 && N % 256 == 0, "gemm_tc_blocked256: N must be a multiple of 256 with 256-wide tiles");
-    static const bool no_tma_store = getenv("OCC_GEMM_NO_TMA_STORE") != nullptr;
-    OCC_CHECK(!(head_major && no_tma_store), "head-major value maps need the TMA-store epilogue");
-    return launch<bf16, false>(A, nullptr, 0, W, bias, nullptr, C, LnArgs{}, M, N, K, ACT_NONE, stream, true, 0, 0, head_major);
+    return launch<bf16, false>(A, nullptr, 0, W, bias, nullptr, C, LnArgs{}, M, N, K, ACT_NONE, stream, true);
 }
 
 // residual, y_f32 and pos are in the T32 block layout (elementwise.cu), rows padded to a multiple of 32
@@ -763,8 +727,8 @@ int gemm_tc_ln(const bf16* A, const bf16* W, const float* bias, const float* res
     GemmProbs probs;
     probs.n = 1;
     int smem = 0;
-    if (build_prob<float, true>(probs.p[0], smem, A, nullptr, 0, W, bias, residual, (float*)nullptr, M, 256, K, ACT_NONE, false, 0, 0, false,
-                                0, 0)) return 1;
+    if (build_prob<float, true>(probs.p[0], smem, A, nullptr, 0, W, bias, residual, (float*)nullptr, M, 256, K, ACT_NONE, false, 0, 0, 0, 0))
+        return 1;
     // the bf16 copies of the LayerNorm output leave through TMA stores of [32 rows x 32 columns]
     probs.p[0].tmC2 = probs.p[0].tmC;
     if (y_bf16 && cached_map_out(y_bf16, 256, (uint64_t)M, 1, 32u, &probs.p[0].tmC)) return 1;
@@ -791,18 +755,17 @@ int gemm_tc_tsa_inputs(const bf16* const* Av, int nv, const bf16* Wv, const floa
     probs.n = nv + 1;
     int smem = 0, sm = 0, begin = 0;
     for (int i = 0; i < nv; ++i) {
-        if (build_prob<bf16, false>(probs.p[i], sm, Av[i], nullptr, 0, Wv, bv, nullptr, Cv[i], M, 256, 256, ACT_NONE, false, 0, 0,
-                                    false, cv, begin)) return 1;
+        if (build_prob<bf16, false>(probs.p[i], sm, Av[i], nullptr, 0, Wv, bv, nullptr, Cv[i], M, 256, 256, ACT_NONE, false, 0, 0, cv,
+                                    begin)) return 1;
         begin += probs.p[i].cta_count;
         smem = sm > smem ? sm : smem;
     }
     // (built through the bf16 instantiation: out_half selects the fp16 packing at run time)
     // rq_t32: the epilogue constant in the T32 layout -> the projection leaves through the TMA-store epilogue as well (the
     // row-major fp32 `rq` forces the staged per-lane epilogue: 4.2-5.5 us per tile instead of 2.1, in-kernel timeline r2 call 8)
-    static const bool no_tma_store = getenv("OCC_GEMM_NO_TMA_STORE") != nullptr;
-    const bool t32 = rq_t32 != nullptr && !no_tma_store && M % 32 == 0;
+    const bool t32 = rq_t32 != nullptr && M % 32 == 0;
     if (build_prob<bf16, false>(probs.p[nv], sm, Aq, Aq2, K1q, Wq, bq, t32 ? nullptr : rq, reinterpret_cast<bf16*>(Cq), M, Nq, Kq,
-                                ACT_NONE, false, 0, 0, false, cq, begin)) return 1;
+                                ACT_NONE, false, 0, 0, cq, begin)) return 1;
     probs.p[nv].out_half = 1;
     if (t32) {
         OCC_CHECK(probs.p[nv].c_tma == 1 && probs.p[nv].stg_bytes == 2048, "gemm_tc_tsa_inputs: T32 constant needs the 32-column TMA-store epilogue");

@@ -19,10 +19,7 @@ int gemm_tc_ln(const bf16* A, const bf16* W, const float* bias, const float* res
 
 // C = A.W^T + bias with N = n*256: output written as n separate contiguous [M,256] bf16 matrices (C + i*M*256).
 // Used to project the camera tokens with the value_proj weights of ALL encoder layers in one pass over the tokens.
-// head_major: every [M,256] block is instead written as 8 head planes [head][M][32] (one 64-byte row per (head, token)):
-// the layout the pair-fetch gather kernel reads (both x-neighbours of a head's bilinear sample are adjacent in memory).
-int gemm_tc_blocked256(const bf16* A, const bf16* W, const float* bias, bf16* C, int M, int N, int K, cudaStream_t stream,
-                       bool head_major = false);
+int gemm_tc_blocked256(const bf16* A, const bf16* W, const float* bias, bf16* C, int M, int N, int K, cudaStream_t stream);
 
 // TemporalSelfAttention's input projections in ONE launch (independent problems on disjoint CTAs): value_proj of 1-2 queue
 // entries (bf16 [M,256]) + the concatenated sampling_offsets / attention_weights projection (fp16 [M,Nq], optional fp32
@@ -30,24 +27,6 @@ int gemm_tc_blocked256(const bf16* A, const bf16* W, const float* bias, bf16* C,
 int gemm_tc_tsa_inputs(const bf16* const* Av, int nv, const bf16* Wv, const float* bv, bf16* const* Cv, const bf16* Aq,
                        const bf16* Aq2, int K1q, const bf16* Wq, const float* bq, const float* rq, const float* rq_t32, __half* Cq,
                        int M, int Nq, int Kq, cudaStream_t stream);
-
-// ---- chained launch (gemm_chain.cu): a list of row-wise independent dense ops executed by ONE persistent kernel; a CTA keeps
-// its row range and an op marked `dep` consumes, tile by tile, what the previous op of the list wrote
-constexpr int GEMM_CHAIN_MAX_OPS = 6;
-struct GemmChainOp {
-    const bf16* A; const bf16* A2; int K1;                   // A = [A (K1 columns) | A2 (K - K1 columns)], A2 may be null (K1 = K)
-    const bf16* W; int N, K;                                 // weights [N, K] bf16
-    const float* bias;                                       // [N] or null
-    int dep;                                                 // A (or A2) rows are written by the previous op of the list
-    // 16-bit output epilogue (ln == 0): C [M, N] bf16 (fp16 if out_half), optional fp32 constant in the T32 layout, activation
-    void* C; int out_half, act; const float* res_t32;
-    // LayerNorm epilogue (ln == 1, N == 256): y = LN(A.W^T + bias + residual); residual / y_f32 / pos in the T32 layout
-    int ln; const float* residual; const float* gamma; const float* beta; const float* pos;
-    float* y_f32; bf16* y_bf16; bf16* y_pos_bf16;
-};
-int gemm_chain_launch(const GemmChainOp* ops, int n_ops, int M, cudaStream_t stream);
-
-int gemm_tc_heads256(const bf16* A, const bf16* W, const float* bias, bf16* C, int M, int K, cudaStream_t stream);
 
 // fp32-grade product of an fp32 operand (given as its bf16 split S = [hi | lo], [M, 2*Ks]) with fp32 weights (given as
 // W3 = [W_hi | W_hi | W_lo], [N, 3*Ks] bf16): 3 tensor-core passes in one launch, relative error ~2^-16.

@@ -26,13 +26,7 @@ int launch_tsa_fused(const T* value_prev, const T* value_cur, const void* qproj,
                      T* out, cudaStream_t stream);
 template <typename T>
 int launch_sca_fused(const T* value, const void* qproj, bool qproj_is_half, const ScaParams& sp, const LevelGeom& lg, int Nv,
-                     T* out, uint8_t* hits, cudaStream_t stream, unsigned* sched = nullptr);
-constexpr int SCA_SCHED_WORDS = 1024;       // scheduler words of the SM-tiled gather kernels: one per %smid + the global tile counter
-int launch_tsa_pair(const bf16* value_prev_hm, const bf16* value_cur_hm, const void* qproj, bool qproj_is_half, int bev_h,
-                    int bev_w, bf16* out, cudaStream_t stream);
-// same gather on head-major value maps [8 heads][num_cams*Nv tokens][32] (pair-fetch kernel, bf16 production path)
-int launch_sca_pair(const bf16* value_hm, const void* qproj, bool qproj_is_half, const ScaParams& sp, const LevelGeom& lg,
-                    int Nv, bf16* out, uint8_t* hits, cudaStream_t stream);
+                     T* out, uint8_t* hits, cudaStream_t stream);
 int launch_project_pillars(const ScaParams& sp, float* ref_cam, uint8_t* mask, cudaStream_t stream);
 
 // ---- backbone_kernels.cu (image backbone + neck, channels-last; first version, see the file header)

@@ -15,7 +15,7 @@
 // a lane accumulates 8 of the head's 32 channels, so one warp-wide 128-bit load instruction
 // fetches 8 independent 64-byte (bf16) corner rows.  Per-sample scalars (location, weight) are
 // prepared by one owner lane per (head, level).
-//   sca_fused_kernel / tsa_fused_kernel (fp32 parity path, bf16 fallback): the owner's packed
+//   sca_fused_kernel (fp32 parity path) / tsa_fused_kernel (both value types): the owner's packed
 //        sample is broadcast inside the 4-lane group with shuffles.
 //   sca_pipe_kernel (bf16 production path): the owners write 16-byte sample descriptors to shared
 //        memory; the gather loop reads them with one broadcast LDS.128 per sample and issues the
@@ -24,8 +24,6 @@
 // Measured bound (ncu, profiles/README.md): the L1 data path -- every 128-bit warp load touches 6-8
 // different 128-byte lines and replays once per line -- not HBM (11 % dram) or instruction issue (50 %).
 #include <cuda_fp16.h>
-
-#include <cstdlib>
 
 #include "common.cuh"
 #include "kernels.cuh"
@@ -294,14 +292,18 @@ __device__ __forceinline__ uint4 make_desc(const SamplePrep& sm)
     return make_uint4((uint32_t)sm.code, pack_bf16x2(sm.c1, sm.c2), pack_bf16x2(sm.c3, sm.c4), 0u);
 }
 
-// one BEV query per warp (the body of both production kernels below); dw = this warp's 4 KB descriptor block
-// getq() returns the query index: the body is register-tight (80 = 6 CTAs/SM) and must be able to RE-DERIVE q where it is used
-// (linear kernel: from blockIdx; SM-tiled kernel: re-read from shared memory) instead of keeping it live across the gather.
-template <typename QT, int DEPTH, typename GetQ>
-__device__ __forceinline__ void sca_pipe_query(GetQ getq, const bf16* __restrict__ value, const QT* __restrict__ qproj,
-                                               const ScaParams& sp, const LevelGeom& lg, int Nv, bf16* __restrict__ out,
-                                               uint8_t* __restrict__ hits, uint4* dw)
+// bf16 production kernel: one BEV query per warp, CTA b = queries [b*NW, (b+1)*NW) in BEV raster order.
+// The body is register-tight (80 = 6 CTAs/SM): getq() RE-DERIVES the query index from blockIdx where it is used instead of
+// keeping it live across the gather.
+template <typename QT, int DEPTH, int MINB, int NW>
+__global__ void __launch_bounds__(NW * 32, MINB)
+sca_pipe_kernel(const bf16* __restrict__ value, const QT* __restrict__ qproj, ScaParams sp, LevelGeom lg,
+                int Nv, bf16* __restrict__ out, uint8_t* __restrict__ hits)
 {
+    __shared__ uint4 descs[NW][32 * 8];                          // [warp][sample = point*4 + level][head ^ swizzle]
+    auto getq = [] { return (int)(blockIdx.x * NW + (threadIdx.x >> 5)); };
+    if (getq() >= sp.bev_h * sp.bev_w) return;
+    uint4* dw = descs[threadIdx.x >> 5];                         // this warp's 4 KB descriptor block
     const int lane = threadIdx.x & 31, head = lane >> 2, s = lane & 3;   // s doubles as the owned level
     const unsigned FULL = 0xffffffffu;
 
@@ -372,226 +374,6 @@ __device__ __forceinline__ void sca_pipe_query(GetQ getq, const bf16* __restrict
 #pragma unroll
     for (int i = 0; i < 8; ++i) acc[i] = __fdiv_rn(acc[i], scale);
     store8(out + (int64_t)getq() * 256 + head * 32 + s * 8, acc);
-}
-
-// Linear mapping: CTA b = queries [b*NW, (b+1)*NW) in BEV raster order (kept as the A/B reference: OCC_SCA_TILED=0).
-template <typename QT, int DEPTH, int MINB, int NW>
-__global__ void __launch_bounds__(NW * 32, MINB)
-sca_pipe_kernel(const bf16* __restrict__ value, const QT* __restrict__ qproj, ScaParams sp, LevelGeom lg,
-                int Nv, bf16* __restrict__ out, uint8_t* __restrict__ hits)
-{
-    __shared__ uint4 descs[NW][32 * 8];                          // [warp][sample = point*4 + level][head ^ swizzle]
-    auto getq = [] { return (int)(blockIdx.x * NW + (threadIdx.x >> 5)); };
-    if (getq() >= sp.bev_h * sp.bev_w) return;
-    sca_pipe_query<QT, DEPTH>(getq, value, qproj, sp, lg, Nv, out, hits, descs[threadIdx.x >> 5]);
-}
-
-// ------------------------------------------------------------------------------------------
-// SM-tiled persistent variant (EXPERIMENT, off by default: measured slower, see launch_sca_fused).  Hypothesis: the gather is
-// bound by L2 -> L1 traffic (ncu, linear mapping: 1.48 GB per launch over the crossbar at 6.5 TB/s, L1 hit rate 47 %, DRAM 8 %):
-// neighbouring BEV queries project onto overlapping image regions, but consecutive CTAs of a linear grid land on DIFFERENT SMs,
-// so the 24 warps resident on an SM work on 6 unrelated strips.
-// Here every SM works on ONE compact BEV tile (TW x TH = 8 x 3 queries = 6 units of 4 x-consecutive queries) at a time:
-//   * grid = #SMs x MINB persistent CTAs of 4 warps; a CTA reads %smid and takes the next unit of its SM's current tile from
-//     one 32-bit word per SM:  word = (tile + 1) << 16 | c;  old = atomicAdd(word, 1), c = old & 0xffff:
-//        tile set, c in [2, U]            -> unit c - 1 of that tile
-//        (no tile, c == 0) or c == U + 1  -> this CTA fetches the SM's next tile t = atomicAdd(global, 1), takes its unit 0 and
-//                                            publishes word = (t + 1) << 16 | 2  (t >= number of tiles: word = DONE)
-//        otherwise                        -> another CTA of this SM is fetching: retry
-//     All-zero words (one cudaMemsetAsync per launch) are the initial state.  Balance is dynamic at tile granularity and no
-//     assumption is made about which / how many CTAs the hardware places on an SM.
-//   * tools/dev/sca_l1_sim.py (LRU model of the bench geometry): L2 -> L1 bytes 1.16 GB -> 0.5-0.6 GB per launch.
-constexpr int SCA_TILE_W = 8, SCA_TILE_H = 3, SCA_TILE_UNITS = (SCA_TILE_W / 4) * SCA_TILE_H;
-constexpr unsigned SCA_TILE_DONE = 0xffffu;
-
-// next unit of this SM's current tile -> first query of the unit (4 x-consecutive queries), -1 = all tiles done, -2 = the unit
-// lies outside the BEV grid.  Kept out of line: nothing of the scheduler stays live across the (register-tight) query body.
-__device__ __noinline__ int sca_tile_next(unsigned* __restrict__ sched, int sched_global, int bev_w, int bev_h)
-{
-    unsigned smid;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    unsigned* word = sched + min(smid, (unsigned)sched_global - 1);
-    const int tiles_x = (bev_w + SCA_TILE_W - 1) / SCA_TILE_W, tiles_y = (bev_h + SCA_TILE_H - 1) / SCA_TILE_H;
-    const unsigned num_tiles = (unsigned)(tiles_x * tiles_y);
-    unsigned tile, unit;
-    for (;;) {
-        const unsigned old = atomicAdd(word, 1u);
-        const unsigned tf = old >> 16, c = old & 0xffffu;            // tf = current tile + 1 (0: none yet)
-        if (tf == SCA_TILE_DONE) return -1;
-        if (tf != 0 && c >= 2 && c <= (unsigned)SCA_TILE_UNITS) { tile = tf - 1; unit = c - 1; break; }
-        if (tf == 0 ? c == 0 : c == (unsigned)SCA_TILE_UNITS + 1) {
-            const unsigned t = atomicAdd(sched + sched_global, 1u);
-            if (t >= num_tiles) { atomicExch(word, (SCA_TILE_DONE << 16) | 8u); return -1; }
-            atomicExch(word, ((t + 1) << 16) | 2u);
-            tile = t; unit = 0;
-            break;
-        }
-        __nanosleep(64);                                             // another CTA of this SM is publishing the next tile
-    }
-    const int x = (int)(tile % tiles_x) * SCA_TILE_W + (int)(unit % (SCA_TILE_W / 4)) * 4;
-    const int y = (int)(tile / tiles_x) * SCA_TILE_H + (int)(unit / (SCA_TILE_W / 4));
-    return (y < bev_h && x < bev_w) ? y * bev_w + x : -2;
-}
-
-template <typename QT, int DEPTH, int MINB>
-__global__ void __launch_bounds__(128, MINB)
-sca_tile_kernel(const bf16* __restrict__ value, const QT* __restrict__ qproj, ScaParams sp, LevelGeom lg,
-                int Nv, bf16* __restrict__ out, uint8_t* __restrict__ hits, unsigned* __restrict__ sched /* [max smid + 1] + global */,
-                int sched_global)
-{
-    __shared__ uint4 descs[4][32 * 8];
-    __shared__ int s_q[2];                                       // double-buffered: one __syncthreads per unit
-    int it = 0;
-    if (threadIdx.x == 0) s_q[0] = sca_tile_next(sched, sched_global, sp.bev_w, sp.bev_h);
-    for (;; it ^= 1) {
-        __syncthreads();
-        const int q0 = s_q[it];
-        if (q0 == -1) return;
-        // the unit after this one is fetched now (atomic round trip hidden behind this unit's gather)
-        if (threadIdx.x == 0) s_q[it ^ 1] = sca_tile_next(sched, sched_global, sp.bev_w, sp.bev_h);
-        const volatile int* sq = &s_q[it];
-        auto getq = [sq] { return *sq + (int)(threadIdx.x >> 5); };   // re-read, not kept live (see sca_pipe_query)
-        if (q0 >= 0)                                                 // (bev_w % 4 == 0: a unit of 4 queries never wraps a row)
-            sca_pipe_query<QT, DEPTH>(getq, value, qproj, sp, lg, Nv, out, hits, descs[threadIdx.x >> 5]);
-    }
-}
-
-// ------------------------------------------------------------------------------------------
-// Pair-fetch variant of the production gather (head-major value maps, written by the value_proj GEMM's TMA-store epilogue):
-//   value_hm [8 heads][T = num_cams * Nv tokens][32] bf16 -- one 64-byte row per (head, token), so the two x-neighbours of a
-//   bilinear sample are ADJACENT: 8 lanes fetch the 128 contiguous bytes {left pixel | right pixel} of one (head, row) with
-//   one 128-bit load each, and a warp instruction covers 4 heads x 128 B.  A sample costs 2 such instructions per head group
-//   (upper row, lower row) instead of 4 corner instructions of 8 x 64 B: the same bytes in half as many 128-byte lines when
-//   the pair is line-aligned (even token), three quarters on average -- the row-major layout touched one line per (head,
-//   corner), and the kernel is bound by L1 lines per request (profiles/README.md).
-//   Lane map in phase 2: hl = lane / 8 (head within the group of 4), j = lane % 8: side = j / 4 (left / right pixel),
-//   slice = j % 4 (8 channels).  Two head groups -> 2 x 8 accumulators per lane; left and right partial sums are combined
-//   with one shuffle per accumulator at the end.  Phase 1 (descriptors) is the row-major kernel's.
-// hack (timing experiments only, results are garbage): 1 = every pair forced onto an even token (line-aligned fetches with
-// the real footprint), 2 = token pitch 128 B (line-aligned fetches with the footprint of a duplicated-pair layout)
-template <int NS, int DEPTH, typename Geom>
-__device__ __forceinline__ void gather_descs_pair(float (&acc)[8], const uint4* dsm, int head, int side, Geom geom, int hack = 0,
-                                                  int64_t tok0 = 0)
-{
-    uint4 d[DEPTH + 1];
-    uint4 v[DEPTH + 1][2];
-    const int pitch = hack == 2 ? 64 : 32;
-#pragma unroll
-    for (int i = 0; i < NS + DEPTH; ++i) {
-        if (i < NS) {
-            const int slot = i % (DEPTH + 1);
-            d[slot] = dsm[desc_slot(i, head)];
-            const bf16* base; int W;
-            geom(i, base, W);
-            if (d[slot].x & CODE_VALID) {
-                int64_t tok = tok0 + (int64_t)(d[slot].x & CODE_OFF_MASK);
-                if (hack == 1) tok &= ~(int64_t)1;
-                const bf16* p = base + tok * pitch;
-                v[slot][0] = __ldg(reinterpret_cast<const uint4*>(p));
-                v[slot][1] = __ldg(reinterpret_cast<const uint4*>(p + (int64_t)W * pitch));
-            }
-        }
-        if (i >= DEPTH) {
-            const int slot = (i - DEPTH) % (DEPTH + 1);
-            if (d[slot].x & CODE_VALID) {
-                const uint32_t w0 = side ? (d[slot].y >> 16) : d[slot].y;     // upper row: right / left corner weight
-                const uint32_t w1 = side ? (d[slot].z >> 16) : d[slot].z;     // lower row
-                fma_word4(acc, v[slot][0], w0); fma_word4(acc, v[slot][1], w1);
-            }
-        }
-    }
-}
-
-template <typename QT, int DEPTH, int MINB, int NW>
-__global__ void __launch_bounds__(NW * 32, MINB)
-sca_pair_kernel(const bf16* __restrict__ value_hm, const QT* __restrict__ qproj, ScaParams sp, LevelGeom lg, int Nv,
-                long long T, bf16* __restrict__ out, uint8_t* __restrict__ hits, int hack)
-{
-    __shared__ uint4 descs[NW][32 * 8];                          // [warp][sample = point*4 + level][head]
-    const int Nq = sp.bev_h * sp.bev_w;
-    const int q = blockIdx.x * NW + (threadIdx.x >> 5);
-    if (q >= Nq) return;
-    const int lane = threadIdx.x & 31, head = lane >> 2, s = lane & 3;   // phase-1 roles: (head, owned level)
-    const int hl = lane >> 3, j = lane & 7, side = j >> 2;               // phase-2 roles
-    const unsigned FULL = 0xffffffffu;
-
-    const float xs = __fdiv_rn((float)(q % sp.bev_w) + 0.5f, (float)sp.bev_w);
-    const float ys = __fdiv_rn((float)(q / sp.bev_w) + 0.5f, (float)sp.bev_h);
-    float ru[2], rv[2];
-    unsigned vis = 0;
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-        const int c = r * 4 + (lane >> 3), z = lane & 7;
-        bool ok = false;
-        ru[r] = 0.f; rv[r] = 0.f;
-        if (c < sp.num_cams && z < sp.D) project_point(sp.cam_mat[c], xs, ys, sp.zs[z], sp, ru[r], rv[r], ok);
-        const unsigned b = __ballot_sync(FULL, ok);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) if ((b >> (8 * k)) & 0xffu) vis |= 1u << (r * 4 + k);
-    }
-    const int count = __popc(vis);
-    if (hits && lane == 0) hits[q] = (uint8_t)count;
-
-    float acc0[8], acc1[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { acc0[i] = 0.f; acc1[i] = 0.f; }
-    uint4* dw = descs[threadIdx.x >> 5];
-    const int own_W = s == 0 ? lg.w[0] : s == 1 ? lg.w[1] : s == 2 ? lg.w[2] : lg.w[3];
-    const int own_H = s == 0 ? lg.h[0] : s == 1 ? lg.h[1] : s == 2 ? lg.h[2] : lg.h[3];
-    const int own_start = s == 0 ? lg.start[0] : s == 1 ? lg.start[1] : s == 2 ? lg.start[2] : lg.start[3];
-    const float own_w = (float)own_W, own_h = (float)own_H;
-
-    for (int c = 0; c < sp.num_cams; ++c) {
-        if (!((vis >> c) & 1u)) continue;                                // warp-uniform
-        {
-            const QT* qp = qproj + (int64_t)q * 768;
-            float off[16], wl[8];
-            load_q<16>(qp + head * 64 + s * 16, off);
-            load_q<8>(qp + 512 + head * 32 + s * 8, wl);
-            float mx = wl[0];
-#pragma unroll
-            for (int i = 1; i < 8; ++i) mx = fmaxf(mx, wl[i]);
-            mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, 1));
-            mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, 2));
-            float sum = 0.f;
-#pragma unroll
-            for (int i = 0; i < 8; ++i) { wl[i] = __expf(wl[i] - mx); sum += wl[i]; }
-            sum += __shfl_xor_sync(FULL, sum, 1);
-            sum += __shfl_xor_sync(FULL, sum, 2);
-            const float inv = __fdividef(1.f, sum);
-            const int r = c >> 2;
-#pragma unroll
-            for (int p = 0; p < 8; ++p) {
-                const int asrc = (c & 3) * 8 + (p % sp.D);               // Z-anchor interleave (:366-373)
-                const float u = __shfl_sync(FULL, r ? ru[1] : ru[0], asrc);
-                const float v = __shfl_sync(FULL, r ? rv[1] : rv[0], asrc);
-                const float w_im = fmaf(u, own_w, off[2 * p] - 0.5f);
-                const float h_im = fmaf(v, own_h, off[2 * p + 1] - 0.5f);
-                dw[desc_slot(p * 4 + s, head)] = make_desc(prep_sample(h_im, w_im, wl[p] * inv, own_H, own_W, own_start));
-            }
-        }
-        __syncwarp();
-        // value_hm + (head * T + cam * Nv) * 32 + j * 8: lanes j = 0..7 of a head read 128 contiguous bytes
-        const int64_t hstride = T * (hack == 2 ? 64 : 32);               // elements per head plane
-        const bf16* v0 = value_hm + (int64_t)hl * hstride + j * 8;
-        const bf16* v1 = v0 + 4 * hstride;
-        const int64_t tok0 = (int64_t)c * Nv;
-        gather_descs_pair<32, DEPTH>(acc0, dw, hl, side, [&](int i, const bf16*& base, int& W) { base = v0; W = lg.w[i & 3]; }, hack, tok0);
-        gather_descs_pair<32, DEPTH>(acc1, dw, 4 + hl, side, [&](int i, const bf16*& base, int& W) { base = v1; W = lg.w[i & 3]; }, hack, tok0);
-        __syncwarp();
-    }
-    const float scale = (float)max(count, 1);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        acc0[i] += __shfl_xor_sync(FULL, acc0[i], 4);                    // left-pixel lanes + right-pixel lanes
-        acc1[i] += __shfl_xor_sync(FULL, acc1[i], 4);
-    }
-    if (side == 0) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { acc0[i] = __fdiv_rn(acc0[i], scale); acc1[i] = __fdiv_rn(acc1[i], scale); }
-        store8(out + (int64_t)q * 256 + hl * 32 + j * 8, acc0);
-        store8(out + (int64_t)q * 256 + (4 + hl) * 32 + j * 8, acc1);
-    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -699,65 +481,6 @@ tsa_fused_kernel(const T* __restrict__ value_prev, const T* __restrict__ value_c
     float acc[8];
     accu.finish(acc, 0.5f, false);
     store8(out + (int64_t)q * 256 + head * 32 + s * 8, acc);
-}
-
-// ------------------------------------------------------------------------------------------
-// Pair-fetch variant of the temporal gather on head-major value maps [8 heads][Nq][32] bf16 (see sca_pair_kernel):
-// phase 1: lane (head, s) prepares its two samples (queue s/2, points 2(s%2), 2(s%2)+1) as shared-memory descriptors
-// [sample = queue*4 + point][head]; phase 2: lane (hl, side, slice) gathers {left | right} pixel pairs for heads hl, 4+hl.
-template <typename QT>
-__global__ void __launch_bounds__(256)
-tsa_pair_kernel(const bf16* __restrict__ value_prev_hm, const bf16* __restrict__ value_cur_hm, const QT* __restrict__ qproj,
-                int bev_h, int bev_w, bf16* __restrict__ out)
-{
-    __shared__ uint4 descs[8][8 * 8];                            // [warp][sample][head]
-    const int q = blockIdx.x * 8 + (threadIdx.x >> 5);
-    const int Nq = bev_h * bev_w;
-    if (q >= Nq) return;
-    const int lane = threadIdx.x & 31, head = lane >> 2, s = lane & 3;
-    const int hl = lane >> 3, j = lane & 7, side = j >> 2;
-    const int qu_own = s >> 1, p0 = (s & 1) * 2;
-    const QT* qp = qproj + (int64_t)q * 192;
-    float offv[4], lgv[2];
-    load_q<4>(qp + head * 16 + qu_own * 8 + p0 * 2, offv);
-    load_q<2>(qp + 128 + head * 8 + qu_own * 4 + p0, lgv);
-    float mx = fmaxf(lgv[0], lgv[1]);
-    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-    const float e0 = expf(lgv[0] - mx), e1 = expf(lgv[1] - mx);
-    float sum = e0 + e1;
-    sum += __shfl_xor_sync(0xffffffffu, sum, 1);
-    const float wt0 = e0 / sum, wt1 = e1 / sum;
-    const float fw = (float)bev_w, fh = (float)bev_h;
-    const float rx = __fdiv_rn((float)(q % bev_w) + 0.5f, fw);
-    const float ry = __fdiv_rn((float)(q / bev_w) + 0.5f, fh);
-    const float wim0 = __fadd_rn(rx, __fdiv_rn(offv[0], fw)) * fw - 0.5f;
-    const float him0 = __fadd_rn(ry, __fdiv_rn(offv[1], fh)) * fh - 0.5f;
-    const float wim1 = __fadd_rn(rx, __fdiv_rn(offv[2], fw)) * fw - 0.5f;
-    const float him1 = __fadd_rn(ry, __fdiv_rn(offv[3], fh)) * fh - 0.5f;
-    uint4* dw = descs[threadIdx.x >> 5];
-    dw[desc_slot(qu_own * 4 + p0, head)] = make_desc(prep_sample(him0, wim0, wt0, bev_h, bev_w));
-    dw[desc_slot(qu_own * 4 + p0 + 1, head)] = make_desc(prep_sample(him1, wim1, wt1, bev_h, bev_w));
-    __syncwarp();
-    float acc0[8], acc1[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { acc0[i] = 0.f; acc1[i] = 0.f; }
-    const int64_t plane = (int64_t)Nq * 32;
-    const bf16* p0v = value_prev_hm + (int64_t)hl * plane + j * 8;
-    const bf16* c0v = value_cur_hm + (int64_t)hl * plane + j * 8;
-    gather_descs_pair<8, 2>(acc0, dw, hl, side, [&](int i, const bf16*& base, int& W) { base = i < 4 ? p0v : c0v; W = bev_w; });
-    gather_descs_pair<8, 2>(acc1, dw, 4 + hl, side,
-                            [&](int i, const bf16*& base, int& W) { base = (i < 4 ? p0v : c0v) + 4 * plane; W = bev_w; });
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        acc0[i] += __shfl_xor_sync(0xffffffffu, acc0[i], 4);
-        acc1[i] += __shfl_xor_sync(0xffffffffu, acc1[i], 4);
-    }
-    if (side == 0) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { acc0[i] *= 0.5f; acc1[i] *= 0.5f; }
-        store8(out + (int64_t)q * 256 + hl * 32 + j * 8, acc0);
-        store8(out + (int64_t)q * 256 + (4 + hl) * 32 + j * 8, acc1);
-    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -926,104 +649,29 @@ int launch_tsa_fused(const T* value_prev, const T* value_cur, const void* qproj,
 template int launch_tsa_fused<float>(const float*, const float*, const void*, bool, int, int, float*, cudaStream_t);
 template int launch_tsa_fused<bf16>(const bf16*, const bf16*, const void*, bool, int, int, bf16*, cudaStream_t);
 
-static int num_sms_here()                                            // per device: one process may drive several GPUs
-{
-    static int cache[64] = {0};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
-    if (cache[dev] == 0) cudaDeviceGetAttribute(&cache[dev], cudaDevAttrMultiProcessorCount, dev);
-    return cache[dev] > 0 ? cache[dev] : 148;
-}
-
 template <typename T>
 int launch_sca_fused(const T* value, const void* qproj_v, bool q_half, const ScaParams& sp, const LevelGeom& lg, int Nv,
-                     T* out, uint8_t* hits, cudaStream_t stream, unsigned* sched)
+                     T* out, uint8_t* hits, cudaStream_t stream)
 {
     OCC_CHECK(lg.num_levels == 4 && sp.num_cams <= 8 && sp.D <= 8 && sp.D >= 1 && 8 % sp.D == 0,
               "sca_fused: supports 4 levels, <= 8 cameras, pillar anchors in {1,2,4,8}");
     for (int l = 0; l < 4; ++l) OCC_CHECK(lg.h[l] >= 2 && lg.w[l] >= 2, "sca_fused: every level must be at least 2x2");
     const int Nq = sp.bev_h * sp.bev_w;
-    const dim3 grid(ceil_div(Nq, 8));
     if constexpr (sizeof(T) == 2) {
-        // production bf16 kernel: descriptor-staged gather, 4 warps per CTA, 6 CTAs per SM (OCC_SCA_PIPE=0: the
-        // shuffle-broadcast kernel that is also the fp32 path; measured variants: profiles/README.md)
-        static const int pipe = getenv("OCC_SCA_PIPE") ? atoi(getenv("OCC_SCA_PIPE")) : 416;
-        // OCC_SCA_TILED=6|5: the SM-tiled persistent kernel (6 / 5 CTAs per SM).  MEASURED SLOWER than the linear mapping although it
-        // does what it was built for (ncu, r2 calls 5-6: L1 hit rate 47 -> 64 %, L2->L1 bytes 1.48 -> 1.03 GB, shared-memory
-        // wavefronts -44 %): 268-282 us vs 225 us per launch -- the gather is not bound by L2->L1 bytes (profiles/README.md).
-        static const int tiled = getenv("OCC_SCA_TILED") ? atoi(getenv("OCC_SCA_TILED")) : 0;
-        if (tiled && sched != nullptr && sp.bev_w % 4 == 0) {
-            // SM-tiled persistent kernel: one word per SM (indexed by %smid, < SCA_SCHED_WORDS - 1) + the global tile counter
-            OCC_CUDA(cudaMemsetAsync(sched, 0, SCA_SCHED_WORDS * sizeof(unsigned), stream));
-            // tiled = 6: 6 CTAs/SM (80 registers, ~40 spilled words per query); 5: 5 CTAs/SM (96 registers, none)
-            const int per_sm = tiled == 5 ? 5 : 6;
-            const int grid = num_sms_here() * per_sm;
-            if (q_half) {
-                if (per_sm == 5) sca_tile_kernel<__half, 1, 5><<<grid, 128, 0, stream>>>(value, (const __half*)qproj_v, sp, lg, Nv, out, hits, sched, SCA_SCHED_WORDS - 1);
-                else             sca_tile_kernel<__half, 1, 6><<<grid, 128, 0, stream>>>(value, (const __half*)qproj_v, sp, lg, Nv, out, hits, sched, SCA_SCHED_WORDS - 1);
-            } else {
-                sca_tile_kernel<float, 1, 6><<<grid, 128, 0, stream>>>(value, (const float*)qproj_v, sp, lg, Nv, out, hits, sched, SCA_SCHED_WORDS - 1);
-            }
-            OCC_CUDA(cudaGetLastError());
-            return 0;
-        }
-        bool done = true;
-#define OCC_SCA_CASE(W, D, B)                                                                                       \
-    case 100 * W + 10 * D + B:                                                                                      \
-        if (q_half) sca_pipe_kernel<__half, D, B, W><<<ceil_div(Nq, W), W * 32, 0, stream>>>(value, (const __half*)qproj_v, sp, lg, Nv, out, hits); \
-        else        sca_pipe_kernel<float, D, B, W><<<ceil_div(Nq, W), W * 32, 0, stream>>>(value, (const float*)qproj_v, sp, lg, Nv, out, hits);  \
-        break;
-        switch (pipe) {
-        OCC_SCA_CASE(4, 1, 6)
-        OCC_SCA_CASE(8, 1, 3)
-        default: done = false;
-        }
-#undef OCC_SCA_CASE
-        if (done) { OCC_CUDA(cudaGetLastError()); return 0; }
+        // production bf16 kernel: descriptor-staged gather, 4 warps per CTA, 6 CTAs per SM (measured variants: profiles/README.md)
+        if (q_half) sca_pipe_kernel<__half, 1, 6, 4><<<ceil_div(Nq, 4), 128, 0, stream>>>(value, (const __half*)qproj_v, sp, lg, Nv, out, hits);
+        else        sca_pipe_kernel<float, 1, 6, 4><<<ceil_div(Nq, 4), 128, 0, stream>>>(value, (const float*)qproj_v, sp, lg, Nv, out, hits);
+    } else {
+        OCC_CHECK(!q_half, "sca_fused: the fp32 kernel reads fp32 projections");
+        sca_fused_kernel<T><<<ceil_div(Nq, 8), 256, 0, stream>>>(value, (const float*)qproj_v, sp, lg, Nv, out, hits);
     }
-    OCC_CHECK(!q_half, "sca_fused: the unpipelined kernel reads fp32 projections");
-    const float* qproj = (const float*)qproj_v;
-    sca_fused_kernel<T><<<grid, 256, 0, stream>>>(value, qproj, sp, lg, Nv, out, hits);
     OCC_CUDA(cudaGetLastError());
     return 0;
 }
 template int launch_sca_fused<float>(const float*, const void*, bool, const ScaParams&, const LevelGeom&, int, float*,
-                                     uint8_t*, cudaStream_t, unsigned*);
+                                     uint8_t*, cudaStream_t);
 template int launch_sca_fused<bf16>(const bf16*, const void*, bool, const ScaParams&, const LevelGeom&, int, bf16*,
-                                    uint8_t*, cudaStream_t, unsigned*);
-
-int launch_tsa_pair(const bf16* value_prev_hm, const bf16* value_cur_hm, const void* qproj, bool q_half, int bev_h, int bev_w,
-                    bf16* out, cudaStream_t stream)
-{
-    OCC_CHECK(bev_h >= 2 && bev_w >= 2, "tsa_pair: the BEV grid must be at least 2x2");
-    const dim3 grid(ceil_div(bev_h * bev_w, 8));
-    if (q_half) tsa_pair_kernel<__half><<<grid, 256, 0, stream>>>(value_prev_hm, value_cur_hm, (const __half*)qproj, bev_h, bev_w, out);
-    else        tsa_pair_kernel<float><<<grid, 256, 0, stream>>>(value_prev_hm, value_cur_hm, (const float*)qproj, bev_h, bev_w, out);
-    OCC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_sca_pair(const bf16* value_hm, const void* qproj_v, bool q_half, const ScaParams& sp, const LevelGeom& lg, int Nv,
-                    bf16* out, uint8_t* hits, cudaStream_t stream)
-{
-    OCC_CHECK(lg.num_levels == 4 && sp.num_cams <= 8 && sp.D <= 8 && sp.D >= 1 && 8 % sp.D == 0,
-              "sca_pair: supports 4 levels, <= 8 cameras, pillar anchors in {1,2,4,8}");
-    for (int l = 0; l < 4; ++l) OCC_CHECK(lg.h[l] >= 2 && lg.w[l] >= 2, "sca_pair: every level must be at least 2x2");
-    const int Nq = sp.bev_h * sp.bev_w;
-    const long long T = (long long)sp.num_cams * Nv;
-    // 6 CTAs/SM caps the kernel at 80 registers (a few spills outside the gather loop); OCC_SCA_PAIR_MINB=5 trades occupancy
-    // for none (measured variants: profiles/README.md)
-    static const int minb = getenv("OCC_SCA_PAIR_MINB") ? atoi(getenv("OCC_SCA_PAIR_MINB")) : 6;
-    static const int hack = getenv("OCC_PAIR_HACK") ? atoi(getenv("OCC_PAIR_HACK")) : 0;     // timing experiments only
-    if (q_half) {
-        if (minb == 5) sca_pair_kernel<__half, 1, 5, 4><<<ceil_div(Nq, 4), 128, 0, stream>>>(value_hm, (const __half*)qproj_v, sp, lg, Nv, T, out, hits, hack);
-        else           sca_pair_kernel<__half, 1, 6, 4><<<ceil_div(Nq, 4), 128, 0, stream>>>(value_hm, (const __half*)qproj_v, sp, lg, Nv, T, out, hits, hack);
-    } else {
-        sca_pair_kernel<float, 1, 6, 4><<<ceil_div(Nq, 4), 128, 0, stream>>>(value_hm, (const float*)qproj_v, sp, lg, Nv, T, out, hits, hack);
-    }
-    OCC_CUDA(cudaGetLastError());
-    return 0;
-}
+                                    uint8_t*, cudaStream_t);
 
 int launch_project_pillars(const ScaParams& sp, float* ref_cam, uint8_t* mask, cudaStream_t stream)
 {

@@ -744,31 +744,6 @@ def test_voxel_lift_from_t32_layout_is_bit_identical():
         assert torch.equal(a[k], b[k]), k
 
 
-def test_chained_dense_layers_are_bit_identical():
-    """OCC_GEMM_CHAIN=1 (gemm_chain.cu: the dense layers between two gathers as ONE persistent launch, a CTA walking the op list
-    over its own rows with per-tile completion counters) against one launch per layer (gemm_tc.cu): same MMA order, same epilogue
-    arithmetic -> bit-identical outputs, without and with a previous BEV, and fewer launches."""
-    code = r"""
-import os, sys, torch
-sys.path.insert(0, 'tests')
-import test_gpu_parity as t
-cfg, params, feats, metas, prev = t.make_case('small6', with_prev=True)
-fd = [f[0].to(t.DEV) for f in feats]
-a = t.engine_for(cfg, params, metas, 'bf16', tc=True)
-os.environ['OCC_GEMM_CHAIN'] = '1'
-b = t.engine_for(cfg, params, metas, 'bf16', tc=True)
-for pb in (None, prev):
-    for rep in range(2):
-        oa = a.forward(fd, prev_bev=pb); la = a.launches_per_frame
-        ob = b.forward(fd, prev_bev=pb); lb = b.launches_per_frame
-        for k in oa:
-            assert torch.equal(oa[k], ob[k]), (k, pb is None, rep)
-    assert lb < la, (la, lb)
-print('OK')
-"""
-    assert 'OK' in _run_isolated(code)
-
-
 def test_layer0_tsa_constant_fold_is_bit_identical():
     """Self mode (prev_bev None): layer 0's TemporalSelfAttention + LayerNorm depend on parameters only and are computed once
     at finalize by the frame path's own kernels; an engine built with OCC_NO_L0_FOLD=1 recomputes them every frame.

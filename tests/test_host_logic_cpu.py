@@ -1,6 +1,6 @@
 """Host-side logic added in round 2, checked without a GPU: the T32 block layout for any column count (mirror of the CUDA tiler
-and of the GEMM epilogue's read), the per-SM tile scheduler word protocol of the experimental SM-tiled gather, the committed
-profile summaries (regenerated from the committed raw ncu export), and the submission writer's argument checks."""
+and of the GEMM epilogue's read), the committed profile summaries (regenerated from the committed raw ncu export), and the
+submission writer's argument checks."""
 import json
 import os
 import subprocess
@@ -23,7 +23,7 @@ def test_t32_layout_is_a_permutation_and_matches_the_epilogue_read(ncols):
     rows = 96
     idx = np.array([[_t32_index(r, c, ncols) for c in range(ncols)] for r in range(rows)])
     assert sorted(idx.reshape(-1)) == list(range(rows * ncols))                    # a permutation of the padded matrix
-    # gemm_tc.cu / gemm_chain.cu epilogue: thread `lane` of the warp that owns rows row0..row0+31 reads, for the 32-column chunk
+    # gemm_tc.cu epilogue: thread `lane` of the warp that owns rows row0..row0+31 reads, for the 32-column chunk
     # starting at column col, the float4s  ((row0 >> 5) * (N >> 5) + (col >> 5)) * 256 + lane + j * 32,  j = 0..7
     for row0 in (0, 32, 64):
         for col in range(0, ncols, 32):
@@ -35,69 +35,6 @@ def test_t32_layout_is_a_permutation_and_matches_the_epilogue_read(ncols):
     # a warp instruction (fixed j) touches 32 consecutive float4 = 512 contiguous bytes: the point of the layout
     lane_addr = [(((0 >> 5) * (ncols >> 5) + 0) * 256 + lane + 3 * 32) for lane in range(32)]
     assert lane_addr == list(range(lane_addr[0], lane_addr[0] + 32))
-
-
-def _sched_step(word, global_tile, num_tiles, units=6, done=0xFFFF):
-    """One `atomicAdd(word, 1)` of msda.cu: sca_tile_next.  Returns (new word, new global counter, outcome) with outcome one of
-    ('unit', tile, unit), ('retry',), ('done',)."""
-    old = word
-    word = (word + 1) & 0xFFFFFFFF
-    tf, c = old >> 16, old & 0xFFFF
-    if tf == done:
-        return word, global_tile, ('done',)
-    if tf != 0 and 2 <= c <= units:
-        return word, global_tile, ('unit', tf - 1, c - 1)
-    if (c == 0) if tf == 0 else (c == units + 1):
-        t = global_tile
-        global_tile += 1
-        if t >= num_tiles:
-            return (done << 16) | 8, global_tile, ('done',)
-        return ((t + 1) << 16) | 2, global_tile, ('unit', t, 0)      # (the exchange happens later on the GPU: see below)
-    return word, global_tile, ('retry',)
-
-
-def test_sm_tile_scheduler_hands_out_every_unit_exactly_once():
-    """Sequentially consistent emulation of the per-SM word protocol with several SMs and CTAs arriving in random order, including
-    arrivals between a fetcher's atomicAdd and its exchange (modelled by a pending exchange that later arrivals see as `retry`)."""
-    rng = np.random.RandomState(0)
-    num_tiles, units, n_sm = 37, 6, 5
-    words, pending = [0] * n_sm, [None] * n_sm
-    g = 0
-    got, live = [], [[True] * 6 for _ in range(n_sm)]
-    steps = 0
-    while any(any(l) for l in live):
-        steps += 1
-        assert steps < 200000
-        sm = rng.randint(n_sm)
-        if pending[sm] is not None and rng.rand() < 0.5:             # the fetcher's atomicExch lands now
-            words[sm] = pending[sm]; pending[sm] = None
-            continue
-        ctas = [i for i, l in enumerate(live[sm]) if l]
-        if not ctas:
-            continue
-        cta = ctas[rng.randint(len(ctas))]
-        if pending[sm] is not None:                                   # word still holds the incremented counter: others retry
-            old = words[sm]; words[sm] = (old + 1) & 0xFFFFFFFF
-            tf, c = old >> 16, old & 0xFFFF
-            assert not (tf != 0 and 2 <= c <= units) and not ((c == 0) if tf == 0 else (c == units + 1)), (tf, c)
-            continue
-        before = words[sm]
-        new_word, g, out = _sched_step(words[sm], g, num_tiles, units)
-        if out[0] == 'unit' and out[2] == 0:                          # a fetch: counter incremented now, exchange deferred
-            words[sm] = (before + 1) & 0xFFFFFFFF
-            pending[sm] = new_word
-            got.append(out[1:])
-        elif out[0] == 'unit':
-            words[sm] = new_word; got.append(out[1:])
-        elif out[0] == 'done':
-            if new_word >> 16 == 0xFFFF and before >> 16 != 0xFFFF:
-                words[sm] = (before + 1) & 0xFFFFFFFF; pending[sm] = new_word
-            else:
-                words[sm] = new_word
-            live[sm][cta] = False
-        else:
-            words[sm] = new_word
-    assert sorted(got) == [(t, u) for t in range(num_tiles) for u in range(units)]
 
 
 def test_committed_profile_summaries_regenerate_from_the_committed_raw_export(tmp_path):
@@ -168,35 +105,3 @@ def test_pack_transpose_swizzle_is_conflict_free_and_consistent():
     for p in range(64):
         pieces = sorted(addr(p, c8) * 2 // 16 for c8 in range(0, 64, 8))
         assert pieces == list(range(p * 8, p * 8 + 8))
-
-
-def test_chain_kernel_completion_protocol_never_publishes_an_incomplete_tile():
-    """gemm_chain.cu: an op whose rows feed the next op publishes tile completions WITHOUT waiting on its freshest stores: after
-    tile t the issuing lane waits until at most `groups(t)` of its bulk store groups are pending (cp.async.bulk.wait_group) and
-    publishes tile t-1; after the last tile it waits for everything and publishes the last one.  Model: 8 epilogue warps, bulk
-    groups complete in FIFO order per warp at random times; the consumer may load tile t once the counter reaches 8 * (t + 1)."""
-    rng = np.random.RandomState(1)
-    for trial in range(200):
-        n_tiles = int(rng.randint(1, 5))
-        groups_per_tile = [[int(rng.choice([0, 3, 4, 8])) for _ in range(n_tiles)] for _ in range(8)]   # 0: warp inactive for the tile
-        done_counter = 0
-        published_when = {}                                       # tile -> list of (warp, groups of that tile all complete?)
-        for w in range(8):
-            committed = []                                        # tile index of every committed group, in order
-            completed = 0                                         # groups completed so far (FIFO)
-            for t in range(n_tiles):
-                committed += [t] * groups_per_tile[w][t]
-                completed = min(len(committed), completed + int(rng.randint(0, 6)))     # some older groups finish meanwhile
-                if t > 0:
-                    pending_allowed = groups_per_tile[w][t]
-                    completed = max(completed, len(committed) - pending_allowed)          # wait_group(pending_allowed)
-                    ok = all(i < completed for i, tt in enumerate(committed) if tt <= t - 1)
-                    published_when.setdefault(t - 1, []).append(ok)
-                    done_counter += 1
-                if t == n_tiles - 1:
-                    completed = len(committed)                                            # wait_group 0
-                    published_when.setdefault(t, []).append(True)
-                    done_counter += 1
-        assert done_counter == 8 * n_tiles
-        for t in range(n_tiles):
-            assert len(published_when[t]) == 8 and all(published_when[t]), (trial, t, groups_per_tile)

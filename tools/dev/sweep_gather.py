@@ -1,6 +1,6 @@
 """Dev aid (not a test): time one engine configuration (env knobs are read at first launch) and print
 ms/frame + per-category ms, plus max |diff| of occ logits against a reference run saved by the first call.
-  python tools/dev/sweep_gather.py TAG   (env: OCC_SCA_PIPE, OCC_TSA_DEPTH, OCC_QPROJ_F32, ...)"""
+  python tools/dev/sweep_gather.py TAG   (env: OCC_NO_L0_FOLD, OCC_GEMM_TIMELINE, OCC_TEST_OFFSCALE)"""
 import json, os, sys
 import numpy as np
 import torch

@@ -573,6 +573,10 @@ int occb200_engine_create(const occb200_config* cfg, occb200_engine** out)
     OCC_CHECK(cfg->pillar_h == 16 && cfg->out_dim == 32, "only pillar_h=16, out_dim=32 are supported");
     OCC_CHECK(cfg->ffn_dim % 64 == 0 && cfg->num_classes <= 32 && cfg->num_layers >= 1, "bad ffn_dim/num_classes");
     OCC_CHECK(cfg->precision == 0 || cfg->precision == 1, "precision must be 0 (fp32) or 1 (bf16)");
+    // the TSA / SCA gathers fetch 2x2 pixel blocks: a side of 1 has none (refused here, not at the first forward)
+    OCC_CHECK(cfg->bev_h >= 2 && cfg->bev_w >= 2, "the BEV grid must be at least 2x2");
+    for (int l = 0; l < 4; ++l)
+        OCC_CHECK(cfg->level_h[l] >= 2 && cfg->level_w[l] >= 2, "every feature level must be at least 2x2");
     int dev_count = 0;
     if (cudaGetDeviceCount(&dev_count) != cudaSuccess || dev_count == 0) {
         set_last_error("no CUDA device: libocc_b200 has no CPU fallback");

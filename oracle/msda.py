@@ -50,39 +50,40 @@ def msda_grid_sample(value, value_spatial_shapes, sampling_locations, attention_
     return out.view(bs, num_heads * embed_dims, num_queries).transpose(1, 2).contiguous()
 
 
-def msda_loops(value, value_spatial_shapes, level_start_index, sampling_locations, attention_weights):
-    """Scalar (numpy, fp32) statement of the CUDA kernel's arithmetic; small cases only."""
-    v = value.detach().cpu().numpy().astype(np.float32)
-    loc = sampling_locations.detach().cpu().numpy().astype(np.float32)
-    aw = attention_weights.detach().cpu().numpy().astype(np.float32)
+def msda_loops(value, value_spatial_shapes, level_start_index, sampling_locations, attention_weights, dtype=np.float32):
+    """Scalar (numpy) statement of the CUDA kernel's arithmetic; small cases only.  `dtype` np.float32 restates the
+    kernel's fp32 rounding, np.float64 gives the operator's value to ~1e-15."""
+    v = value.detach().cpu().numpy().astype(dtype)
+    loc = sampling_locations.detach().cpu().numpy().astype(dtype)
+    aw = attention_weights.detach().cpu().numpy().astype(dtype)
     B, Nv, M, C = v.shape
     _, Nq, _, L, P, _ = loc.shape
-    out = np.zeros((B, Nq, M, C), np.float32)
-    f32 = np.float32
+    out = np.zeros((B, Nq, M, C), dtype)
+    fl = np.dtype(dtype).type
     for b in range(B):
         for q in range(Nq):
             for m in range(M):
-                acc = np.zeros(C, np.float32)
+                acc = np.zeros(C, dtype)
                 for l in range(L):
                     H = int(value_spatial_shapes[l][0]); W = int(value_spatial_shapes[l][1])
                     base = int(level_start_index[l])
                     for p in range(P):
-                        w_im = f32(loc[b, q, m, l, p, 0] * f32(W) - f32(0.5))
-                        h_im = f32(loc[b, q, m, l, p, 1] * f32(H) - f32(0.5))
+                        w_im = fl(loc[b, q, m, l, p, 0] * fl(W) - fl(0.5))
+                        h_im = fl(loc[b, q, m, l, p, 1] * fl(H) - fl(0.5))
                         if not (h_im > -1 and w_im > -1 and h_im < H and w_im < W):
                             continue
                         h_lo = int(np.floor(h_im)); w_lo = int(np.floor(w_im))
-                        lh = f32(h_im - f32(h_lo)); lw = f32(w_im - f32(w_lo))
-                        hh = f32(1) - lh; hw = f32(1) - lw
-                        val = np.zeros(C, np.float32)
+                        lh = fl(h_im - fl(h_lo)); lw = fl(w_im - fl(w_lo))
+                        hh = fl(1) - lh; hw = fl(1) - lw
+                        val = np.zeros(C, dtype)
                         if h_lo >= 0 and w_lo >= 0:
-                            val += f32(hh * hw) * v[b, base + h_lo * W + w_lo, m]
+                            val += fl(hh * hw) * v[b, base + h_lo * W + w_lo, m]
                         if h_lo >= 0 and w_lo + 1 <= W - 1:
-                            val += f32(hh * lw) * v[b, base + h_lo * W + w_lo + 1, m]
+                            val += fl(hh * lw) * v[b, base + h_lo * W + w_lo + 1, m]
                         if h_lo + 1 <= H - 1 and w_lo >= 0:
-                            val += f32(lh * hw) * v[b, base + (h_lo + 1) * W + w_lo, m]
+                            val += fl(lh * hw) * v[b, base + (h_lo + 1) * W + w_lo, m]
                         if h_lo + 1 <= H - 1 and w_lo + 1 <= W - 1:
-                            val += f32(lh * lw) * v[b, base + (h_lo + 1) * W + w_lo + 1, m]
+                            val += fl(lh * lw) * v[b, base + (h_lo + 1) * W + w_lo + 1, m]
                         acc += aw[b, q, m, l, p] * val
                 out[b, q, m] = acc
     return torch.from_numpy(out.reshape(B, Nq, M * C))
